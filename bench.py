@@ -22,6 +22,8 @@ Timing   : CUDA events on the work stream, max over ranks, barrier + synchronize
            `roofline_ransac` the FP64-bound RANSAC kernel.  Peak = MEASURED_PEAKS.json (HBM copy GB/s).
 `clocks` : NVML samples taken by the benchmark thread inside every warm-up and timed step (see ClockSampler).
 `cpu_baseline` / `--impl reference`: the CPU oracle port (oracle/) on a bounded sample of the same workload.
+`--dump-outputs DIR`: after the timed steps, what the last one computed goes to DIR/<name>.npy (see dump_outputs); the
+           inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -300,6 +302,51 @@ def run_step(clouds, numbers, n_poses_total, w, world, profile=False, read_table
 
 
 # ------------------------------------------------------------------------------------------------
+# --dump-outputs
+# ------------------------------------------------------------------------------------------------
+DUMP_COUNTERS = ("n_points_inserted", "n_points_alive", "n_cells", "n_leaves", "n_internal", "n_blocks", "max_depth_reached")
+DUMP_ROWS = {"leaf": 1 << 18, "plane": 1 << 18, "point": 1 << 19}  # 48 + 56 + 32 B per row: 44 MB at most
+DUMP_SEED = 20240917
+
+
+def _sample_rows(n, k, salt):
+    """sorted indices of a fixed, seeded sample of k of n rows (every row when n <= k)"""
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng([DUMP_SEED, salt]).choice(n, size=k, replace=False))
+
+
+def dump_outputs(grid, out_dir):
+    """Write what a step hands its caller as out_dir/<name>.npy, float64 throughout except the float32 planes:
+      counters           the forest's counters (DUMP_COUNTERS order)
+      pose_counts        (poses, 3) leaves, points, nodes per pose, in insertion order (Grid.n_leaves / n_points / n_nodes)
+      leaf_*             leaf table (corner, edge, cell, depth)
+      plane, plane_*     per-block RANSAC table, reference block order (plane, pose, leaf, size, best, best_count)
+      point_xyz, _idx    surviving points in reference block order, with their index in their pose's cloud
+    The three tables are sampled to at most DUMP_ROWS rows each; the sample depends only on the table's length."""
+    forest = grid._host.forest
+    st = forest.stats()
+    out = {"counters": np.array([st[k] for k in DUMP_COUNTERS], dtype=np.float64),
+           "pose_counts": np.asarray(grid._host.counts(), dtype=np.float64)}
+    leaves = forest.export_leaves()
+    rows = _sample_rows(len(leaves["edge"]), DUMP_ROWS["leaf"], 0)
+    for k in ("corner", "edge", "cell", "depth"):
+        out["leaf_" + k] = leaves[k][rows].astype(np.float64)
+    planes = forest.export_ransac(scored_only=True)
+    rows = _sample_rows(len(planes["plane"]), DUMP_ROWS["plane"], 1)
+    out["plane"] = planes["plane"][rows].astype(np.float32)
+    for k in ("pose", "leaf", "size", "best", "best_count"):
+        out["plane_" + k] = planes[k][rows].astype(np.float64)
+    points = forest.export_points(-1, order=0)
+    rows = _sample_rows(len(points["idx"]), DUMP_ROWS["point"], 2)
+    out["point_xyz"] = points["xyz"][rows].astype(np.float64)
+    out["point_idx"] = points["idx"][rows].astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+# ------------------------------------------------------------------------------------------------
 # CPU baseline / reference arm: the REAL reference (oracle/_ref, made by oracle/make_ref.sh) on a bounded sample
 # ------------------------------------------------------------------------------------------------
 def _sample_clouds(workload, n_sample_points):
@@ -484,6 +531,7 @@ def _claim_stdout():
 
 
 def main():
+    sys.dont_write_bytecode = True  # the benchmark may run from a read-only tree: it writes nothing there
     result_out = _claim_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -496,8 +544,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-full-path", action="store_true", help="skip the clutter workload (RANSAC without early exits)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
     rank, world, local = dist_env()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.impl != "ours" or world > 1):
+        ap.error("--dump-outputs needs --impl ours on one GPU")
     w = WORKLOADS[args.workload]
     cores = os.cpu_count() or 1
     base = {"metric": "points/sec (insert+subdivide+per-leaf RANSAC)", "unit": "points/s", "n_gpus": args.gpus,
@@ -586,6 +639,8 @@ def main():
     ms_per_step = ms / args.steps
     value = total / (ms_per_step * 1e-3)
     stats = res[1]
+    if args.dump_outputs:
+        dump_outputs(res[0], args.dump_outputs)
     del res  # the last timed grid must not stay alive next to the profiled / e2e grids (memory at the 1e9-point scale)
 
     # profiled step (separate from the timed ones): per-stage times for the roofline object, executed-arithmetic tallies of

@@ -14,6 +14,7 @@ from __future__ import annotations
 import ctypes
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -23,10 +24,17 @@ _lib = None
 
 
 def build(force: bool = False) -> str:
-    """Compile oracle/ransac_oracle.c with gcc (see oracle/Makefile)."""
+    """Compile oracle/ransac_oracle.c with gcc (see oracle/Makefile).  In a read-only tree (bench.py may run from
+    one) a stale or missing library is compiled into a temporary directory instead of oracle/_build."""
+    global _LIB_PATH
     src = os.path.join(_HERE, "ransac_oracle.c")
     if force or not os.path.exists(_LIB_PATH) or os.path.getmtime(_LIB_PATH) < os.path.getmtime(src):
-        subprocess.check_call(["make", "-s", "-C", _HERE, "-B"])
+        if os.access(_HERE, os.W_OK):
+            subprocess.check_call(["make", "-s", "-C", _HERE, "-B"])
+        else:
+            out = tempfile.mkdtemp(prefix="ol_oracle_")
+            subprocess.check_call(["make", "-s", "-C", _HERE, "-B", f"BUILD={out}"])
+            _LIB_PATH = os.path.join(out, "libransac_oracle.so")
     return _LIB_PATH
 
 
