@@ -136,11 +136,43 @@ int ol_forest_subdivide_levels(ol_forest *f, const int32_t *first_level, int32_t
                                const uint8_t *split_tables_host, int64_t table_len, const int32_t *split_beyond,
                                const int32_t *pose_indices, int32_t n_poses);
 
+/* Geometric criteria (octreelib_b200/criteria.py: MaxExtent, MaxThickness, Planar).  A term looks at the points a node
+ * holds (the listed poses' points for a subdivision with pose indices), all in float64:
+ *   extent    = max over the axes of (max coordinate - min coordinate), 0 for an empty node;
+ *   thickness = sqrt(max(smallest eigenvalue of the population covariance, 0)), the RMS distance of the points from
+ *               their least-squares plane; 0 for fewer than 3 points.
+ * A term holds iff the node has at least min_points points and  stat > value (OL_GEOM_GT) / stat <= value (OL_GEOM_LE).
+ * The reference evaluates such criteria per node in Python (octree/octree.py:26, :111). */
+#define OL_GEOM_EXTENT 0
+#define OL_GEOM_THICKNESS 1
+#define OL_GEOM_GT 0
+#define OL_GEOM_LE 1
+#define OL_GEOM_MAX_TERMS 8 /* terms per rule entry */
+typedef struct ol_geom_term {
+    int32_t stat;       /* OL_GEOM_EXTENT / OL_GEOM_THICKNESS */
+    int32_t op;         /* OL_GEOM_GT / OL_GEOM_LE */
+    int64_t min_points; /* >= 0 */
+    double value;       /* >= 0 */
+} ol_geom_term;
+
+/* Grid.subdivide with criteria that look at coordinates (octree/octree.py:20-32 with e.g. "split while not planar"):
+ * the arguments of ol_forest_subdivide_levels plus, per entry e, n_terms[e] terms (at most OL_GEOM_MAX_TERMS) stored
+ * back to back in `terms` (entry 0 first).  A node of a level of entry e splits iff the count rule says so OR one of
+ * the entry's terms holds.  Counts as a subdivide call (the leaf order across calls, ol_forest_export_leaves). */
+int ol_forest_subdivide_geometric(ol_forest *f, const int32_t *first_level, int32_t n_entries, const int64_t *level_max_points,
+                                  const uint8_t *split_tables_host, int64_t table_len, const int32_t *split_beyond,
+                                  const ol_geom_term *terms, const int32_t *n_terms, const int32_t *pose_indices,
+                                  int32_t n_poses);
+
 /* ---- Grid.filter, grid/grid.py:260-267 -> octree/octree.py:102-112 --------------------------
  * A (pose, leaf) block of n points survives iff keep_table[min(n, table_len-1)] != 0; the tree
  * shape is unchanged.  n_poses == 0: all poses. */
 int ol_forest_filter(ol_forest *f, const uint8_t *keep_table_host, int64_t table_len, const int32_t *pose_indices,
                      int32_t n_poses);
+/* Same, with geometric terms (octree/octree.py:111, e.g. "keep planar leaves"): a block of a listed pose survives iff
+ * the keep table says so AND all n_terms terms (at most OL_GEOM_MAX_TERMS) hold on its points. */
+int ol_forest_filter_geometric(ol_forest *f, const uint8_t *keep_table_host, int64_t table_len, const ol_geom_term *terms,
+                               int32_t n_terms, const int32_t *pose_indices, int32_t n_poses);
 
 /* ---- Grid.map_leaf_points_cuda_ransac, grid/grid.py:124-215 ---------------------------------
  * table_host: [H][K] float64 uniform [0,1) hypothesis table (ransac/cuda_ransac.py:39-41).
@@ -220,6 +252,12 @@ int ol_forest_export_leaves(ol_forest *f, double *corner, double *edge, int32_t 
 /* non-empty (pose, leaf) blocks in the order Grid.get_leaf_points / the RANSAC batches use
  * (pose rank, then the reference's leaf order for that pose):  pose[B], leaf[B] (index into the leaf table), size[B]. */
 int ol_forest_export_blocks(ol_forest *f, const int32_t *pose_rank, int32_t *pose, int32_t *leaf, int32_t *size);
+/* Point statistics of the same blocks, in the same order, for one pose (pose_index >= 0) or all (-1): what a plane-based
+ * back end reads instead of reducing Grid.get_leaf_points(...)[i].get_points() (grid.py:217-232) leaf by leaf.  Per row:
+ * pose[B], n[B], mean[B][3], cov[B][6] (population covariance xx, xy, xz, yy, yz, zz), extent[B][3] (max - min per axis).
+ * *out_n = number of rows; with every array NULL only *out_n is written. */
+int ol_forest_export_block_stats(ol_forest *f, const int32_t *pose_rank, int32_t pose_index, int32_t *pose, int64_t *n,
+                                 double *mean, double *cov, double *extent, int64_t *out_n);
 /* the block table as it was when ol_forest_ransac last ran (before the masks were applied), same
  * order, plus per block: plane[B][4] float32, best[B] (hypothesis index, -1 = skipped because the
  * block has fewer than K points, ransac/cuda_ransac.py:96-97), best_count[B] (its inlier count).

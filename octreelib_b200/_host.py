@@ -9,7 +9,7 @@ from typing import Callable, Dict, List, Optional, Sequence
 import numpy as np
 
 from . import _views
-from .criteria import CountCriterion, NotCountOnly, as_threshold, fold_count_criteria, fold_levels
+from .criteria import CountCriterion, GeometricCriterion, NotCountOnly, as_threshold, fold_count_criteria, fold_levels
 from .forest import Forest
 
 __all__ = ["ForestHost"]
@@ -87,8 +87,18 @@ class ForestHost:
             self._counts_cache = None
             return
         guarded = any(isinstance(c, CountCriterion) and c.size_guarded for c in criteria)
-        # [(first level, table, beyond, criteria active from that level on)]; one entry unless node-size guards are used
-        levels = fold_levels(criteria, float(self._edge), 1024) if guarded else None
+        # [(first level, table, beyond, count criteria active from that level on, geometric terms)]; one entry unless
+        # node-size guards are used
+        if any(isinstance(c, GeometricCriterion) for c in criteria):
+            try:
+                levels = fold_levels(criteria, float(self._edge), 1024)  # (the geometric objects are not probed)
+            except NotCountOnly:
+                # an opaque criterion next to the geometric ones: the whole list is evaluated on the host
+                self._subdivide_on_host(criteria, idx)
+                self._counts_cache = None
+                return
+        else:
+            levels = fold_levels(criteria, float(self._edge), 1024) if guarded else None
         if levels is None:
             try:
                 table, beyond = fold_count_criteria(criteria, "any", 1024)
@@ -100,11 +110,14 @@ class ForestHost:
                 self._subdivide_on_host(criteria, idx)
                 self._counts_cache = None
                 return
-            levels = [(0, table, beyond, criteria)]
-        thresholds = [as_threshold(t, b, active) if active else (1 << 62) for _, t, b, active in levels]
+            levels = [(0, table, beyond, criteria, [])]
+        thresholds = [as_threshold(t, b, active) if active else (1 << 62) for _, t, b, active, _ in levels]
         firsts = [lv[0] for lv in levels]
+        terms = [lv[4] for lv in levels]
         if all(t is not None for t in thresholds):
-            if len(levels) == 1:
+            if any(terms):
+                self.forest.subdivide_geometric(firsts, terms, thresholds=thresholds, pose_indices=idx)
+            elif len(levels) == 1:
                 self.forest.subdivide(thresholds[0], idx)
             else:
                 self.forest.subdivide_levels(firsts, thresholds=thresholds, pose_indices=idx)
@@ -112,7 +125,7 @@ class ForestHost:
             n_alive = self.forest.stats()["n_points_alive"]
             upto = min(n_alive + 1, _TABLE_CAP)
             tables, beyonds = [], []
-            for _, _, _, active in levels:
+            for _, _, _, active, _ in levels:
                 if active:
                     table, beyond = fold_count_criteria(active, "any", upto)
                 else:
@@ -123,7 +136,9 @@ class ForestHost:
                     beyond = False
                 tables.append(table)
                 beyonds.append(beyond)
-            if len(levels) == 1:
+            if any(terms):
+                self.forest.subdivide_geometric(firsts, terms, tables=tables, beyonds=beyonds, pose_indices=idx)
+            elif len(levels) == 1:
                 self.forest.subdivide_table(tables[0], beyonds[0], idx)
             else:
                 self.forest.subdivide_levels(firsts, tables=tables, beyonds=beyonds, pose_indices=idx)
@@ -134,12 +149,14 @@ class ForestHost:
         if self.empty:
             return
         idx = self._indices(pose_numbers)
-        if any(isinstance(c, CountCriterion) and c.size_guarded for c in criteria):
+        if any(isinstance(c, (CountCriterion, GeometricCriterion)) and c.size_guarded for c in criteria):
             raise NotImplementedError("node-size guards (max_depth / min_edge) apply to subdivision criteria, not to filters")
+        geometric = [c for c in criteria if isinstance(c, GeometricCriterion)]
+        counted = [c for c in criteria if not isinstance(c, GeometricCriterion)] if geometric else criteria
         max_block = self.forest.stats()["max_block_size"]
         upto = min(max_block + 1, _TABLE_CAP)
         try:
-            table, beyond = fold_count_criteria(criteria, "all", upto)
+            table, beyond = fold_count_criteria(counted, "all", upto)
         except NotCountOnly:
             self._filter_on_host(list(criteria), idx)
             self._counts_cache = None
@@ -149,7 +166,10 @@ class ForestHost:
                 raise NotImplementedError("count criterion without a settled answer for very large leaves")
             table[-1] = 1 if beyond else 0
         # an EMPTY leaf is also "filtered" by the reference, which changes nothing
-        self.forest.filter(table, idx)
+        if geometric:
+            self.forest.filter_geometric(table, [c.term() for c in geometric], idx)
+        else:
+            self.forest.filter(table, idx)
         self._counts_cache = None
 
     # ---- opaque (coordinate-dependent) criteria: evaluated on the host like the reference does -------------------------
@@ -313,6 +333,24 @@ class ForestHost:
             keep[j] = True
             j += 1
         return keep
+
+    # ---- per-leaf point statistics ------------------------------------------------------------------
+    def leaf_statistics(self, pose_number: Optional[int] = None) -> dict:
+        """n, mean, covariance (population, (B,3,3)), extent (per axis) and pose number of the non-empty (pose, leaf)
+        blocks: of one pose in `get_leaf_points` order, or of all poses in the RANSAC batch order (pose numbers
+        ascending, then the reference's leaf order).  Computed on the device (ol_forest_export_block_stats)."""
+        if pose_number is not None and pose_number not in self.pose_index:
+            raise KeyError(pose_number)
+        if self.empty:
+            return dict(n=np.zeros(0, np.int64), mean=np.zeros((0, 3)), covariance=np.zeros((0, 3, 3)), extent=np.zeros((0, 3)),
+                        pose=np.zeros(0, np.int64))
+        numbers = np.asarray(self.pose_numbers, dtype=np.int64)
+        rank = np.empty(len(numbers), dtype=np.int32)
+        rank[np.argsort(numbers, kind="stable")] = np.arange(len(numbers), dtype=np.int32)
+        s = self.forest.export_block_stats(-1 if pose_number is None else self.pose_index[pose_number], rank)
+        cov = np.asarray(s["cov"], dtype=np.float64)[:, [0, 1, 2, 1, 3, 4, 2, 4, 5]].reshape(-1, 3, 3)
+        return dict(n=np.asarray(s["n"], dtype=np.int64), mean=np.array(s["mean"], dtype=np.float64), covariance=cov,
+                    extent=np.array(s["extent"], dtype=np.float64), pose=numbers[np.asarray(s["pose"], dtype=np.int64)])
 
     # ---- counters (grid.py:343-362) --------------------------------------------------------------
     def counts(self) -> np.ndarray:

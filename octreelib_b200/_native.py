@@ -46,6 +46,15 @@ class ForestStats(C.Structure):
         "n_blocks", "max_block_size", "max_depth_reached", "key_bits", "device_bytes_peak", "sample_oob_seen")]
 
 
+OL_GEOM_EXTENT, OL_GEOM_THICKNESS = 0, 1
+OL_GEOM_GT, OL_GEOM_LE = 0, 1
+OL_GEOM_MAX_TERMS = 8
+
+
+class GeomTerm(C.Structure):
+    _fields_ = [("stat", C.c_int32), ("op", C.c_int32), ("min_points", C.c_int64), ("value", C.c_double)]
+
+
 class NativeLibraryMissing(ImportError):
     pass
 
@@ -69,6 +78,9 @@ SIGNATURES = {
     "ol_forest_subdivide": (C.c_int, [_p, _i64, _p, _i32]),
     "ol_forest_subdivide_table": (C.c_int, [_p, _p, _i64, _i32, _p, _i32]),
     "ol_forest_subdivide_levels": (C.c_int, [_p, _p, _i32, _p, _p, _i64, _p, _p, _i32]),
+    "ol_forest_subdivide_geometric": (C.c_int, [_p, _p, _i32, _p, _p, _i64, _p, _p, _p, _p, _i32]),
+    "ol_forest_filter_geometric": (C.c_int, [_p, _p, _i64, _p, _i32, _p, _i32]),
+    "ol_forest_export_block_stats": (C.c_int, [_p, _p, _i32, _p, _p, _p, _p, _p, C.POINTER(_i64)]),
     "ol_forest_export_shape": (C.c_int, [_p, _p, _p, _p, C.POINTER(_i64)]),
     "ol_forest_impose_shape": (C.c_int, [_p, _p, _p, _p, _i64]),
     "ol_forest_filter": (C.c_int, [_p, _p, _i64, _p, _i32]),

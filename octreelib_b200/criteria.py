@@ -23,6 +23,17 @@ decision (`level_limit`), evaluated by `decide_kernel`.  Called as a plain calla
 oracle - a guarded criterion reads the edge of the node under test from the caller's frame (`self` of
 `OctreeNode.subdivide`, octree/octree.py:20-32), which makes the very same object usable with the unmodified
 reference: that is how tests/golden/make_golden.py pins the semantics.
+
+Geometric criteria.  `MaxExtent(e)` ("split while the node spans more than e"), `MaxThickness(t)` ("split while the node
+is not planar") and `Planar(t)` ("keep planar leaves") look at the coordinates, through two float64 statistics of the
+points they are handed: the EXTENT (largest per-axis max - min) and the THICKNESS (RMS distance of the points from their
+least-squares plane, sqrt of the smallest eigenvalue of the population covariance).  They are declarative: `subdivide` /
+`filter` evaluate them on the GPU (the per-node statistics are one segmented reduction over the points the level loop
+holds per leaf, csrc/geometry.cuh) without probing, while the same objects remain plain callables for the reference and
+the CPU oracle.  They take the same node-size guards as `MaxPoints` (evaluated by the guard logic of `CountCriterion`).
+Extent decisions agree with numpy bit for bit; thickness decisions agree unless a node's thickness lies within the bound
+documented in csrc/geometry.cuh of the threshold.  A list that also holds an opaque coordinate-dependent callable is
+evaluated on the host as before.
 """
 from __future__ import annotations
 
@@ -32,7 +43,8 @@ from typing import Callable, List, Optional, Sequence, Tuple
 import numpy as np
 
 __all__ = ["MaxPoints", "MinPoints", "MaxDepth", "MinEdge", "CountCriterion", "fold_count_criteria", "as_threshold",
-           "fold_levels", "NO_LEVEL_LIMIT", "NotCountOnly"]
+           "fold_levels", "NO_LEVEL_LIMIT", "NotCountOnly", "GeometricCriterion", "MaxExtent", "MaxThickness", "Planar",
+           "extent", "thickness"]
 
 
 class NotCountOnly(NotImplementedError):
@@ -179,6 +191,113 @@ class MinEdge(CountCriterion):
 
     def __init__(self, edge: float):
         super().__init__(">=", 0, min_edge=edge)
+
+
+def extent(points) -> float:
+    """Largest per-axis extent (max - min) of an (n, 3) cloud, in float64; 0.0 for an empty cloud."""
+    p = np.asarray(points, dtype=np.float64).reshape(-1, 3)
+    if len(p) == 0:
+        return 0.0
+    return float((p.max(axis=0) - p.min(axis=0)).max())
+
+
+def thickness(points) -> float:
+    """RMS distance of the points from their least-squares plane: sqrt(max(smallest eigenvalue of the population
+    covariance, 0)), two-pass in float64; 0.0 for fewer than 3 points."""
+    p = np.asarray(points, dtype=np.float64).reshape(-1, 3)
+    n = len(p)
+    if n < 3:
+        return 0.0
+    d = p - p.mean(axis=0)
+    cov = (d.T @ d) / n
+    return float(np.sqrt(max(float(np.linalg.eigvalsh(cov)[0]), 0.0)))
+
+
+class GeometricCriterion:
+    """`<stat>(points) <op> value` for clouds of at least `min_points` points, stat = 'extent' or 'thickness', op = '>'
+    or '<=', as a callable object with inspectable parameters.  The optional node-size guards `max_depth` / `min_edge`
+    mean what they mean for `MaxPoints`: they are evaluated by a `CountCriterion` guard (level_limit / on_node)."""
+
+    STATS = {"extent": (0, extent), "thickness": (1, thickness)}  # name -> (native code, host definition)
+    OPS = {">": 0, "<=": 1}
+
+    def __init__(self, stat: str, op: str, value: float, min_points: int = 1, max_depth: Optional[int] = None,
+                 min_edge: Optional[float] = None, voxel_edge_length: Optional[float] = None):
+        if stat not in self.STATS:
+            raise ValueError(f"unknown statistic {stat!r}")
+        if op not in self.OPS:
+            raise ValueError(f"unknown comparison {op!r}")
+        value = float(value)
+        if not (np.isfinite(value) and value >= 0):
+            raise ValueError(f"{stat} threshold must be finite and >= 0, got {value}")
+        if int(min_points) < 1:
+            raise ValueError("min_points must be >= 1")
+        self.stat, self.op, self.value, self.min_points = stat, op, value, int(min_points)
+        self._guard = CountCriterion(">=", self.min_points, max_depth, min_edge, voxel_edge_length)
+
+    @property
+    def max_depth(self) -> Optional[int]:
+        return self._guard.max_depth
+
+    @property
+    def min_edge(self) -> Optional[float]:
+        return self._guard.min_edge
+
+    @property
+    def size_guarded(self) -> bool:
+        return self._guard.size_guarded
+
+    def level_limit(self, root_edge: float) -> int:
+        """Nodes at level >= this (cell root = level 0) never satisfy the criterion."""
+        return self._guard.level_limit(root_edge)
+
+    def term(self) -> tuple:
+        """(statistic code, comparison code, min_points, value): one ol_geom_term of the native rule."""
+        return (self.STATS[self.stat][0], self.OPS[self.op], self.min_points, self.value)
+
+    def on_points(self, points) -> bool:
+        """The criterion without its node-size guards."""
+        p = np.asarray(points, dtype=np.float64).reshape(-1, 3)
+        if len(p) < self.min_points:
+            return False
+        v = self.STATS[self.stat][1](p)
+        return v > self.value if self.op == ">" else v <= self.value
+
+    def __call__(self, points) -> bool:
+        if not self.on_points(points):
+            return False
+        if not self.size_guarded:
+            return True
+        return self._guard.on_node(len(points), _edge_of_node_under_test())
+
+    def __repr__(self):
+        guard = "".join(f", {k}={v}" for k, v in (("max_depth", self.max_depth), ("min_edge", self.min_edge)) if v is not None)
+        return f"GeometricCriterion({self.stat}(points) {self.op} {self.value}, min_points={self.min_points}{guard})"
+
+
+class MaxExtent(GeometricCriterion):
+    """Subdivide while a node's points span more than `e` along some axis (max - min); with `max_depth` / `min_edge`
+    only down to that depth / node size."""
+
+    def __init__(self, e: float, max_depth: Optional[int] = None, min_edge: Optional[float] = None,
+                 voxel_edge_length: Optional[float] = None):
+        super().__init__("extent", ">", e, 1, max_depth, min_edge, voxel_edge_length)
+
+
+class MaxThickness(GeometricCriterion):
+    """Subdivide while a node of at least `min_points` points is not planar: its points lie farther than `t` (RMS) from
+    their least-squares plane; with `max_depth` / `min_edge` only down to that depth / node size."""
+
+    def __init__(self, t: float, min_points: int = 4, max_depth: Optional[int] = None, min_edge: Optional[float] = None,
+                 voxel_edge_length: Optional[float] = None):
+        super().__init__("thickness", ">", t, min_points, max_depth, min_edge, voxel_edge_length)
+
+
+class Planar(GeometricCriterion):
+    """Keep a leaf only if it holds at least `min_points` points lying within `t` (RMS) of their least-squares plane."""
+
+    def __init__(self, t: float, min_points: int = 3):
+        super().__init__("thickness", "<=", t, min_points)
 
 
 def _probe(n: int, fill: float) -> np.ndarray:
@@ -342,21 +461,25 @@ def as_threshold(table: np.ndarray, beyond: bool, criteria: Sequence[Callable] =
 
 
 def fold_levels(criteria: Sequence[Callable], root_edge: float, upto: int):
-    """Per-level form of `any(criteria)` for subdivision with node-size guards.
+    """Per-level form of `any(criteria)` for subdivision with node-size guards and geometric criteria.
 
-    Returns a list of (first_level, table, beyond): the decision table that applies from `first_level` on (until the
-    next entry's first level); the last entry applies to every deeper level.  Without guarded criteria the list has one
-    entry that starts at level 0."""
+    Returns a list of (first_level, table, beyond, count criteria, geometric terms): the count decision table and the
+    native terms (GeometricCriterion.term) that apply from `first_level` on (until the next entry's first level); the
+    last entry applies to every deeper level.  A node splits iff the table OR one of the terms says so.  Without guarded
+    criteria the list has one entry that starts at level 0."""
     criteria = list(criteria)
-    limits = [c.level_limit(root_edge) if isinstance(c, CountCriterion) else NO_LEVEL_LIMIT for c in criteria]
+    guarded = (CountCriterion, GeometricCriterion)
+    limits = [c.level_limit(root_edge) if isinstance(c, guarded) else NO_LEVEL_LIMIT for c in criteria]
     cuts = sorted({0} | {l for l in limits if l < NO_LEVEL_LIMIT})
     out = []
     for first in cuts:
         active = [c for c, l in zip(criteria, limits) if l > first]
-        plain = [CountCriterion(c.op, c.n) if isinstance(c, CountCriterion) else c for c in active]
+        plain = [CountCriterion(c.op, c.n) if isinstance(c, CountCriterion) else c for c in active
+                 if not isinstance(c, GeometricCriterion)]
+        terms = [c.term() for c in active if isinstance(c, GeometricCriterion)]
         if plain:
             table, beyond = fold_count_criteria(plain, "any", upto)
         else:
             table, beyond = np.zeros(upto + 1, dtype=np.uint8), False
-        out.append((first, table, beyond, plain))
+        out.append((first, table, beyond, plain, terms))
     return out

@@ -1,5 +1,6 @@
 // extern "C" entry points of liboctreelib_b200 (declared in include/octreelib_b200.h).
 #include <atomic>
+#include <cfloat>
 #include <algorithm>
 #include <new>
 
@@ -199,16 +200,12 @@ int ol_forest_subdivide_table(ol_forest* f, const uint8_t* split_table_host, int
     OL_API_END
 }
 
-int ol_forest_subdivide_levels(ol_forest* f, const int32_t* first_level, int32_t n_entries, const int64_t* level_max_points,
-                               const uint8_t* split_tables_host, int64_t table_len, const int32_t* split_beyond,
-                               const int32_t* pose_indices, int32_t n_poses) {
-    OL_NEED(f);
-    OL_NEED(first_level);
-    OL_API_BEGIN
+// the count part of a level-dependent split rule (ol_forest_subdivide_levels / _geometric)
+static ol::Forest::SplitRule level_rule(const int32_t* first_level, int32_t n_entries, const int64_t* level_max_points,
+                                        const uint8_t* split_tables_host, int64_t table_len, const int32_t* split_beyond) {
     OL_REQUIRE(n_entries >= 1 && n_entries <= 64, OL_ERR_INVALID, "split rule needs 1..64 level entries");
     OL_REQUIRE(split_tables_host ? split_beyond != nullptr : level_max_points != nullptr, OL_ERR_INVALID,
                "split rule needs thresholds or tables");
-    ForestScope scope(f->impl);
     ol::Forest::SplitRule rule;
     for (int e = 0; e < n_entries; ++e) {
         rule.first_level.push_back(first_level[e]);
@@ -223,6 +220,49 @@ int ol_forest_subdivide_levels(ol_forest* f, const int32_t* first_level, int32_t
     }
     rule.tables_host = split_tables_host;
     rule.table_len = split_tables_host ? table_len : 0;
+    return rule;
+}
+
+static void check_geom_terms(const ol_geom_term* terms, int32_t n) {
+    OL_REQUIRE(n >= 0 && n <= OL_GEOM_MAX_TERMS, OL_ERR_INVALID,
+               "at most " + std::to_string(OL_GEOM_MAX_TERMS) + " geometric terms per rule entry");
+    OL_REQUIRE(n == 0 || terms, OL_ERR_INVALID, "NULL geometric terms");
+    for (int32_t t = 0; t < n; ++t) {
+        OL_REQUIRE(terms[t].stat == OL_GEOM_EXTENT || terms[t].stat == OL_GEOM_THICKNESS, OL_ERR_INVALID, "unknown geometric statistic");
+        OL_REQUIRE(terms[t].op == OL_GEOM_GT || terms[t].op == OL_GEOM_LE, OL_ERR_INVALID, "unknown geometric comparison");
+        OL_REQUIRE(terms[t].min_points >= 0, OL_ERR_INVALID, "min_points must be >= 0");
+        OL_REQUIRE(terms[t].value >= 0.0 && terms[t].value <= DBL_MAX, OL_ERR_INVALID, "a geometric threshold must be finite and >= 0");
+    }
+}
+
+int ol_forest_subdivide_levels(ol_forest* f, const int32_t* first_level, int32_t n_entries, const int64_t* level_max_points,
+                               const uint8_t* split_tables_host, int64_t table_len, const int32_t* split_beyond,
+                               const int32_t* pose_indices, int32_t n_poses) {
+    OL_NEED(f);
+    OL_NEED(first_level);
+    OL_API_BEGIN
+    ol::Forest::SplitRule rule = level_rule(first_level, n_entries, level_max_points, split_tables_host, table_len, split_beyond);
+    ForestScope scope(f->impl);
+    f->impl.subdivide(rule, pose_indices, n_poses);
+    OL_API_END
+}
+
+int ol_forest_subdivide_geometric(ol_forest* f, const int32_t* first_level, int32_t n_entries, const int64_t* level_max_points,
+                                  const uint8_t* split_tables_host, int64_t table_len, const int32_t* split_beyond,
+                                  const ol_geom_term* terms, const int32_t* n_terms, const int32_t* pose_indices,
+                                  int32_t n_poses) {
+    OL_NEED(f);
+    OL_NEED(first_level);
+    OL_NEED(n_terms);
+    OL_API_BEGIN
+    ol::Forest::SplitRule rule = level_rule(first_level, n_entries, level_max_points, split_tables_host, table_len, split_beyond);
+    rule.term_begin.push_back(0);
+    for (int e = 0; e < n_entries; ++e) {
+        check_geom_terms(terms ? terms + rule.term_begin.back() : nullptr, n_terms[e]);
+        rule.terms.insert(rule.terms.end(), terms + rule.term_begin.back(), terms + rule.term_begin.back() + n_terms[e]);
+        rule.term_begin.push_back(rule.term_begin.back() + n_terms[e]);
+    }
+    ForestScope scope(f->impl);
     f->impl.subdivide(rule, pose_indices, n_poses);
     OL_API_END
 }
@@ -253,6 +293,17 @@ int ol_forest_filter(ol_forest* f, const uint8_t* keep_table_host, int64_t table
     OL_API_BEGIN
     ForestScope scope(f->impl);
     f->impl.filter(keep_table_host, table_len, pose_indices, n_poses);
+    OL_API_END
+}
+
+int ol_forest_filter_geometric(ol_forest* f, const uint8_t* keep_table_host, int64_t table_len, const ol_geom_term* terms,
+                               int32_t n_terms, const int32_t* pose_indices, int32_t n_poses) {
+    OL_NEED(f);
+    OL_NEED(keep_table_host);
+    OL_API_BEGIN
+    check_geom_terms(terms, n_terms);
+    ForestScope scope(f->impl);
+    f->impl.filter(keep_table_host, table_len, pose_indices, n_poses, terms, n_terms);
     OL_API_END
 }
 
@@ -372,6 +423,16 @@ int ol_forest_export_blocks(ol_forest* f, const int32_t* pose_rank, int32_t* pos
     OL_API_BEGIN
     ForestScope scope(f->impl);
     f->impl.export_blocks(pose_rank, pose, leaf, size);
+    OL_API_END
+}
+
+int ol_forest_export_block_stats(ol_forest* f, const int32_t* pose_rank, int32_t pose_index, int32_t* pose, int64_t* n,
+                                 double* mean, double* cov, double* extent, int64_t* out_n) {
+    OL_NEED(f);
+    OL_NEED(out_n);
+    OL_API_BEGIN
+    ForestScope scope(f->impl);
+    *out_n = f->impl.export_block_stats(pose_rank, pose_index, pose, n, mean, cov, extent);
     OL_API_END
 }
 

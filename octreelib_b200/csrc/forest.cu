@@ -435,6 +435,10 @@ __global__ void mark_alive_kernel(const uint32_t* __restrict__ perm, uint32_t n,
 // =============================================================================================
 // K4: level-synchronous subdivision
 // =============================================================================================
+}  // namespace ol
+#include "geometry.cuh"
+namespace ol {
+
 __global__ void weighted_count_kernel(const uint32_t* __restrict__ leaf_of, const uint32_t* __restrict__ perm,
                                       const uint8_t* __restrict__ ldepth, int level,
                                       const uint32_t* __restrict__ seg_start, const int32_t* __restrict__ seg_pose,
@@ -467,9 +471,11 @@ __host__ __device__ inline uint64_t replay_key(uint32_t cell, uint32_t depth, ui
 // depth: nothing may split, a leaf that wants to is an error.  Template parameters, so that the threshold and table
 // instantiations are straight-line code without stores: the scan evaluates 16 leaves per thread back to back, and only
 // then does the compiler issue the loads of all of them together (with the branches of the other modes in the way every
-// leaf cost its own one or two round trips to memory: 25 us for a scan over 600 k leaves).
+// leaf cost its own one or two round trips to memory: 25 us for a scan over 600 k leaves).  GEOM = the level also has
+// geometric terms (geometry.cuh): a leaf splits if the count rule OR one of the terms says so, evaluated on the leaf's
+// statistics in `geo`; the count-only instantiations never see those loads.
 enum DecideMode { DECIDE_THRESHOLD = 0, DECIDE_TABLE = 1, DECIDE_REPLAY = 2 };
-template <int MODE, bool CAP>
+template <int MODE, bool CAP, bool GEOM = false>
 struct DecideIn {
     const uint32_t* __restrict__ lstart;
     const uint8_t* __restrict__ ldepth;
@@ -485,6 +491,9 @@ struct DecideIn {
     const uint32_t* lcell;
     const uint64_t* lpath;
     uint32_t* err;
+    const GeomLeaf* __restrict__ geo;
+    const ol_geom_term* __restrict__ terms;
+    int n_terms;
     __device__ __forceinline__ uint32_t operator()(size_t k) const {
         bool want = false;
         if (MODE == DECIDE_REPLAY) {
@@ -511,6 +520,10 @@ struct DecideIn {
                 want = cnt < table_len ? (t != 0) : (beyond != 0);
             } else {
                 want = cnt > max_points;
+            }
+            if (GEOM) {
+                const GeomLeaf g = geo[k];
+                for (int t = 0; t < n_terms; ++t) want = want || geom_term_holds(terms[t], g.n, g.extent, g.thickness);
             }
             want = want && (int)depth == level;
             if (CAP) {

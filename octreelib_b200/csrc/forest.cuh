@@ -205,6 +205,24 @@ struct Forest {
         const uint8_t* tables_host = nullptr;  // [entries][table_len]
         int64_t table_len = 0;
         std::vector<int> beyond;
+        // geometric terms (geometry.cuh), OR-ed with the count rule: entry e owns terms[term_begin[e] .. term_begin[e + 1])
+        std::vector<ol_geom_term> terms;
+        std::vector<int> term_begin;  // empty: no entry has terms
+        int n_terms(int e) const { return term_begin.empty() ? 0 : term_begin[e + 1] - term_begin[e]; }
+        bool needs_cov(int e) const {
+            for (int t = 0; t < n_terms(e); ++t)
+                if (terms[term_begin[e] + t].stat == OL_GEOM_THICKNESS) return true;
+            return false;
+        }
+        // fewest points of a node on which a term of entry e can hold (a "> value" term needs at least one point)
+        int64_t geom_min_points(int e) const {
+            int64_t m = INT64_MAX;
+            for (int t = 0; t < n_terms(e); ++t) {
+                const ol_geom_term& g = terms[term_begin[e] + t];
+                m = std::min<int64_t>(m, g.op == OL_GEOM_GT ? std::max<int64_t>(g.min_points, 1) : g.min_points);
+            }
+            return m;
+        }
         int entry_for(int level) const {
             int e = 0;
             for (size_t i = 0; i < first_level.size(); ++i)
@@ -214,7 +232,7 @@ struct Forest {
     };
     void subdivide(const SplitRule& rule, const int32_t* poses, int n_poses_listed);  // K4
     void split_levels(const SplitRule* rule, const uint8_t* d_tables, const uint8_t* d_listed, int n_listed,
-                      const uint64_t* replay_keys, uint32_t n_replay);  // the level loop of K4
+                      const uint64_t* replay_keys, uint32_t n_replay, const ol_geom_term* d_terms = nullptr);  // the level loop of K4
     void reserve_internal(size_t need);
     void ensure_max_block();
     // copies up to 8 small device objects into the pinned scratch block back to back with ONE stream synchronisation
@@ -234,7 +252,10 @@ struct Forest {
     void materialize_order();  // perm / mort / leaf_of := base order, if reset_shape deferred the copy
     void ensure_order();     // K5: leaf enumeration order + geometry
     void ensure_blocks();    // (pose, leaf) runs
-    void filter(const uint8_t* keep_table, int64_t table_len, const int32_t* poses, int n_poses_listed);
+    void filter(const uint8_t* keep_table, int64_t table_len, const int32_t* poses, int n_poses_listed,
+                const ol_geom_term* terms = nullptr, int n_terms = 0);
+    int64_t export_block_stats(const int32_t* pose_rank, int pose, int32_t* o_pose, int64_t* o_n, double* o_mean, double* o_cov,
+                               double* o_ext);
     void apply_keep(const uint8_t* keep_pos);  // K7: drop positions with keep == 0
     void compute_ref_order(const int32_t* pose_rank_host, DevBuf<uint32_t>& ref_order, DevBuf<int32_t>& d_pose_rank,
                            DevBuf<uint32_t>* sorted_rank = nullptr);

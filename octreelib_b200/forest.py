@@ -293,6 +293,29 @@ class Forest:
         self._pending_sources.clear()
         self.version += 1
 
+    def subdivide_geometric(self, first_levels: Sequence[int], terms: Sequence[Sequence[tuple]],
+                            thresholds: Optional[Sequence[int]] = None, tables=None, beyonds: Optional[Sequence[bool]] = None,
+                            pose_indices: Optional[Sequence[int]] = None):
+        """`subdivide_levels` whose entries also carry geometric terms (stat, op, min_points, value), OR-ed with the
+        count rule: terms[e] belongs to the entry that starts at first_levels[e] (`ol_forest_subdivide_geometric`)."""
+        arr, n = _i32_array(pose_indices)
+        fl = np.ascontiguousarray(list(first_levels), dtype=np.int32)
+        flat = [t for entry in terms for t in entry]
+        term_arr = (N.GeomTerm * max(len(flat), 1))(*[N.GeomTerm(int(s), int(o), int(m), float(v)) for s, o, m, v in flat])
+        counts = np.ascontiguousarray([len(entry) for entry in terms], dtype=np.int32)
+        with self._scope():
+            if tables is None:
+                th = np.ascontiguousarray([min(int(t), 1 << 62) for t in thresholds], dtype=np.int64)
+                N.check(self._lib.ol_forest_subdivide_geometric(self._h, _ptr(fl), len(fl), _ptr(th), None, 0, None, term_arr,
+                                                                _ptr(counts), _ptr(arr), n))
+            else:
+                tab = np.ascontiguousarray(np.stack([np.asarray(t, dtype=np.uint8) for t in tables]), dtype=np.uint8)
+                by = np.ascontiguousarray([1 if b else 0 for b in beyonds], dtype=np.int32)
+                N.check(self._lib.ol_forest_subdivide_geometric(self._h, _ptr(fl), len(fl), None, _ptr(tab), tab.shape[1], _ptr(by),
+                                                                term_arr, _ptr(counts), _ptr(arr), n))
+        self._pending_sources.clear()
+        self.version += 1
+
     def export_shape(self) -> dict:
         """The split nodes of the forest: cell coordinates, depth and Morton path (`ol_forest_export_shape`)."""
         n = C.c_int64(0)
@@ -320,6 +343,16 @@ class Forest:
         tab = np.ascontiguousarray(keep_table, dtype=np.uint8)
         with self._scope():
             N.check(self._lib.ol_forest_filter(self._h, _ptr(tab), len(tab), _ptr(arr), n))
+        self.version += 1
+
+    def filter_geometric(self, keep_table: np.ndarray, terms: Sequence[tuple], pose_indices: Optional[Sequence[int]] = None):
+        """`filter` whose blocks must also satisfy every geometric term (stat, op, min_points, value)
+        (`ol_forest_filter_geometric`)."""
+        arr, n = _i32_array(pose_indices)
+        tab = np.ascontiguousarray(keep_table, dtype=np.uint8)
+        term_arr = (N.GeomTerm * max(len(terms), 1))(*[N.GeomTerm(int(s), int(o), int(m), float(v)) for s, o, m, v in terms])
+        with self._scope():
+            N.check(self._lib.ol_forest_filter_geometric(self._h, _ptr(tab), len(tab), term_arr, len(terms), _ptr(arr), n))
         self.version += 1
 
     def ransac(self, table: np.ndarray, threshold: float, pose_rank: Optional[Sequence[int]] = None,
@@ -439,6 +472,23 @@ class Forest:
         with self._scope():
             N.check(self._lib.ol_forest_export_blocks(self._h, _ptr(pr), _ptr(pose), _ptr(leaf), _ptr(size)))
         return dict(pose=pose, leaf=leaf, size=size)
+
+    def export_block_stats(self, pose_index: int = -1, pose_rank: Optional[Sequence[int]] = None) -> dict:
+        """Point statistics of the non-empty (pose, leaf) blocks in `export_blocks` order, of one pose or of all (-1):
+        n, mean (B,3), cov (B,6: xx xy xz yy yz zz, population), extent (B,3) (`ol_forest_export_block_stats`)."""
+        B = self.stats()["n_blocks"]
+        pose = self._host_array(B, np.int32)
+        n = self._host_array(B, np.int64)
+        mean = self._host_array((B, 3), np.float64)
+        cov = self._host_array((B, 6), np.float64)
+        extent = self._host_array((B, 3), np.float64)
+        pr, _ = _i32_array(pose_rank)
+        rows = C.c_int64(0)
+        with self._scope():
+            N.check(self._lib.ol_forest_export_block_stats(self._h, _ptr(pr), int(pose_index), _ptr(pose), _ptr(n), _ptr(mean),
+                                                           _ptr(cov), _ptr(extent), C.byref(rows)))
+        k = rows.value
+        return dict(pose=pose[:k], n=n[:k], mean=mean[:k], cov=cov[:k], extent=extent[:k])
 
     def export_ransac(self, scored_only: bool = False) -> dict:
         """Per-block result table of the last RANSAC run (reference block order)."""

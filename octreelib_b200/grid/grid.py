@@ -111,6 +111,14 @@ class Grid(GridBase):
 
         return host.leaf_voxels(pose_number, non_empty, root_corner, self._grid_config.voxel_edge_length)
 
+    def leaf_statistics(self, pose_number: Optional[int] = None) -> dict:
+        """Point statistics of the non-empty leaves, computed on the GPU: a dict of numpy arrays `n` (B,), `mean` (B, 3),
+        `covariance` (B, 3, 3, population), `extent` (B, 3, max - min per axis) and `pose` (B,, pose numbers).  With a
+        pose number, row i belongs to `get_leaf_points(pose_number)[i]`; without, the rows cover every pose in the order
+        of the RANSAC batches (pose numbers ascending, then the reference's leaf order).  An unknown pose is a KeyError.
+        This is the per-(pose, leaf) hand-off of a plane-based back end (count, centroid, covariance)."""
+        return self._host.leaf_statistics(pose_number)
+
     # ---- grid.py:234-242 ------------------------------------------------------------------------
     def get_points(self, pose_number: int) -> PointCloud:
         return self._host.points_dict_order(pose_number)
