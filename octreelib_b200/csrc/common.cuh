@@ -478,6 +478,23 @@ extern unsigned long long g_mail_ticket;  // last ticket handed out (process-wid
 // waits for the ticket; `stream` is only queried now and then to notice a dead producer
 MailResult mail_wait(const Mail& m, cudaStream_t stream);
 
+#ifdef __CUDACC__
+// Run index of a segmentation, kept by the caller after segment_runs: the head bit of every element (one word per 32)
+// and the number of runs that start before every word.  8 B per 32 elements.
+struct RunIndex {
+    const uint32_t* words;
+    const uint32_t* word_off;
+    const unsigned long long* d_total;
+    uint32_t n;
+    // number of runs that start before element p (p <= n): the run of element p is runs_before(p + 1) - 1, and the runs
+    // of the elements [p, q) are [runs_before(p), runs_before(q)) when p is a head
+    __device__ __forceinline__ uint32_t runs_before(uint32_t p) const {
+        if (p >= n) return (uint32_t)*d_total;
+        return word_off[p >> 5] + __popc(words[p >> 5] & ((1u << (p & 31)) - 1u));
+    }
+};
+#endif
+
 // RAII device buffer of T, bound to a Ctx.
 template <typename T>
 struct DevBuf {

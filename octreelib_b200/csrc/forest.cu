@@ -293,9 +293,12 @@ struct GroupPoseKeyFn {  // (group of the position, pose of its point): group = 
     const uint32_t* seg_start;
     const int32_t* seg_pose;
     int n_seg;
-    __device__ uint64_t operator()(uint32_t i) const {
-        return ((uint64_t)group[i] << 32) | (uint64_t)(uint32_t)seg_pose[seg_of_rank(seg_start, n_seg, perm[i])];
+    // two stages (primitives.cuh: RunKey): (group, rank) from the coalesced arrays, then the pose of the rank
+    __device__ __forceinline__ uint64_t load(uint32_t i) const { return ((uint64_t)group[i] << 32) | (uint64_t)perm[i]; }
+    __device__ __forceinline__ uint64_t finish(uint64_t v) const {
+        return (v & 0xffffffff00000000ull) | (uint64_t)(uint32_t)seg_pose[seg_of_rank(seg_start, n_seg, (uint32_t)v)];
     }
+    __device__ uint64_t operator()(uint32_t i) const { return finish(load(i)); }
 };
 struct CellPoseEmitFn {  // (cell, pose) pairs that own an octree; the first pose of a cell created it (dict order, grid.py:56)
     uint32_t* cp_cell;
@@ -1098,6 +1101,11 @@ __global__ void block_keep_kernel(uint32_t nb, const uint32_t* __restrict__ blk_
         keep = table[sz];
     }
     keep_blk[b] = keep;
+}
+
+__global__ void run_of_pos_kernel(RunIndex ri, uint32_t n, uint32_t* __restrict__ run_of_pos) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) run_of_pos[i] = ri.runs_before(i + 1) - 1u;
 }
 
 __global__ void pos_keep_from_block_kernel(uint32_t n, const uint32_t* __restrict__ blk_of_pos,

@@ -152,7 +152,12 @@ struct Forest {
     DevBuf<uint32_t> blk_start;  // [NB+1] position of the block's first point
     DevBuf<uint32_t> blk_leaf;   // [NB] DFS leaf index
     DevBuf<int32_t> blk_pose;    // [NB]
-    DevBuf<uint32_t> blk_of_pos; // [A] position -> block
+    DevBuf<uint32_t> blk_words;     // [(A + 31) / 32] block-head bit of every position
+    DevBuf<uint32_t> blk_word_off;  // [(A + 31) / 32] blocks that start before every word of blk_words
+    RunIndex blk_index() const { return RunIndex{blk_words.get(), blk_word_off.get(), d_nb.get(), A}; }
+    DevBuf<uint32_t> blk_of_pos; // [A] position -> block, derived from the run index on demand (ensure_blk_of_pos)
+    bool blk_of_pos_valid = false;
+    void ensure_blk_of_pos();
     uint32_t max_block = 0;
     bool max_block_known = false;  // max_block holds the size of the largest block
     bool max_block_enqueued = false;  // ... or a kernel that leaves it in d_max_block has been launched

@@ -5,6 +5,8 @@
 #include "common.cuh"
 #include "onesweep.cuh"
 
+#include <type_traits>
+
 namespace ol {
 
 // =============================================================================================
@@ -434,6 +436,20 @@ constexpr int RUNS_THREADS = 256;
 constexpr int RUNS_ITEMS = 8;
 constexpr int RUNS_TILE = RUNS_THREADS * RUNS_ITEMS;
 
+// A key functor may come in two stages: `load(i)` (the element's own coalesced loads) and `finish(loaded)` (what
+// depends on them, e.g. a table search).  The kernels then issue the loads of all RUNS_ITEMS elements of a thread
+// before the first search: with one stage, a search between two elements kept one DRAM load per thread in flight.
+template <typename KeyFn, typename = void>
+struct RunKey {
+    static __device__ __forceinline__ uint64_t load(const KeyFn& k, uint32_t i) { return k(i); }
+    static __device__ __forceinline__ uint64_t finish(const KeyFn&, uint64_t v) { return v; }
+};
+template <typename KeyFn>
+struct RunKey<KeyFn, std::void_t<decltype(&KeyFn::finish)>> {
+    static __device__ __forceinline__ uint64_t load(const KeyFn& k, uint32_t i) { return k.load(i); }
+    static __device__ __forceinline__ uint64_t finish(const KeyFn& k, uint64_t v) { return k.finish(v); }
+};
+
 template <typename KeyFn>
 __device__ __forceinline__ void runs_warp_flags(const KeyFn& key, uint32_t wbase, uint32_t n, int lane, uint32_t masks[RUNS_ITEMS],
                                                 uint64_t keys[RUNS_ITEMS]) {
@@ -448,8 +464,11 @@ __device__ __forceinline__ void runs_warp_flags(const KeyFn& key, uint32_t wbase
 #pragma unroll
     for (int j = 0; j < RUNS_ITEMS; ++j) {
         const uint32_t i = wbase + 32 * j + lane;
-        keys[j] = i < n ? key(i) : 0ull;
+        keys[j] = i < n ? RunKey<KeyFn>::load(key, i) : 0ull;
     }
+#pragma unroll
+    for (int j = 0; j < RUNS_ITEMS; ++j)
+        if (wbase + 32 * j + lane < n) keys[j] = RunKey<KeyFn>::finish(key, keys[j]);
 #pragma unroll
     for (int j = 0; j < RUNS_ITEMS; ++j) {
         const uint32_t i = wbase + 32 * j + lane;
@@ -557,7 +576,8 @@ __global__ void __launch_bounds__(RUNS_THREADS) runs_emit2_kernel(KeyFn key, Emi
                                                                   const uint32_t* __restrict__ flag_words,
                                                                   const uint32_t* __restrict__ tile_off,
                                                                   const unsigned long long* __restrict__ d_total,
-                                                                  uint32_t* __restrict__ run_of_pos, uint32_t* __restrict__ sentinel) {
+                                                                  uint32_t* __restrict__ run_of_pos, uint32_t* __restrict__ sentinel,
+                                                                  uint32_t* __restrict__ word_off) {
     __shared__ uint32_t s_w[RUNS_THREADS / 32];
     const uint32_t tile = blockIdx.x;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -576,14 +596,21 @@ __global__ void __launch_bounds__(RUNS_THREADS) runs_emit2_kernel(KeyFn key, Emi
     for (int w = 0; w < RUNS_THREADS / 32; ++w)
         if (w < warp) run += s_w[w];
     const uint32_t lt = (1u << lane) - 1u;
+    uint64_t loaded[RUNS_ITEMS];  // the heads' key loads first, all in flight together (RunKey)
+#pragma unroll
+    for (int j = 0; j < RUNS_ITEMS; ++j) {
+        const uint32_t i = wbase + 32 * j + lane;
+        loaded[j] = i < n && ((masks[j] >> lane) & 1u) ? RunKey<KeyFn>::load(key, i) : 0ull;
+    }
 #pragma unroll
     for (int j = 0; j < RUNS_ITEMS; ++j) {
         const uint32_t i = wbase + 32 * j + lane;
         const bool head = (masks[j] >> lane) & 1u;
         const uint32_t mine = run + __popc(masks[j] & lt) + (head ? 1u : 0u) - 1u;
+        if (word_off && lane == j && wbase + 32 * j < n) word_off[(wbase >> 5) + j] = run;
         if (i < n) {
             if (run_of_pos) run_of_pos[i] = mine;
-            if (head) emit(mine, i, key(i));
+            if (head) emit(mine, i, RunKey<KeyFn>::finish(key, loaded[j]));
         }
         run += __popc(masks[j]);
     }
@@ -595,21 +622,28 @@ constexpr size_t RUNS_TWO_PASS_MIN = (size_t)1 << 20;
 // (may be nullptr) and the number of runs to d_total (device, 64-bit).  Run tables must hold the caller's upper bound.
 // `sentinel` (may be nullptr): a run-start table whose entry [number of runs] is set to n by the kernel itself, so that
 // the host does not have to know the count to close the table.  `mail`: the count posted to the host (common.cuh).
+// `words` / `word_off` (both or neither; (n + 31) / 32 entries each): the caller keeps the run index (common.cuh: RunIndex);
+// the two-pass form then runs for every n.
 template <typename KeyFn, typename EmitFn>
 inline void segment_runs(Ctx& c, KeyFn key, EmitFn emit, size_t n, uint32_t* run_of_pos, unsigned long long* d_total,
-                         uint32_t* sentinel = nullptr, const Mail& mail = Mail{}) {
+                         uint32_t* sentinel = nullptr, const Mail& mail = Mail{}, uint32_t* words = nullptr,
+                         uint32_t* word_off = nullptr) {
     OL_REQUIRE(n > 0, OL_ERR_INTERNAL, "segment_runs: empty input");
     const size_t tiles = (n + RUNS_TILE - 1) / RUNS_TILE;
     static const bool one_pass = getenv("OL_RUNS_ONE_PASS") != nullptr;  // debug / A-B: the chained kernel for every size
-    if (n >= RUNS_TWO_PASS_MIN && !one_pass) {
+    if ((n >= RUNS_TWO_PASS_MIN && !one_pass) || words) {
         OL_REQUIRE(d_total != nullptr, OL_ERR_INTERNAL, "segment_runs: the two-pass form needs a device total");
-        DevBuf<uint32_t> flag_words(c, (n + 31) / 32), tile_cnt(c, tiles);
-        runs_flags_kernel<KeyFn><<<(unsigned)tiles, RUNS_THREADS, 0, c.stream>>>(key, (uint32_t)n, flag_words.get(), tile_cnt.get());
+        DevBuf<uint32_t> own_words, tile_cnt(c, tiles);
+        if (!words) {
+            own_words.reset(c, (n + 31) / 32);
+            words = own_words.get();
+        }
+        runs_flags_kernel<KeyFn><<<(unsigned)tiles, RUNS_THREADS, 0, c.stream>>>(key, (uint32_t)n, words, tile_cnt.get());
         OL_CHECK_LAUNCH();
         transform_scan<uint32_t>(c, ScanPtrIn<uint32_t>{tile_cnt.get()}, ScanPtrOut<uint32_t>{tile_cnt.get()}, tiles, d_total, "scan", mail);
         runs_emit2_kernel<KeyFn, EmitFn><<<(unsigned)tiles, RUNS_THREADS, 0, c.stream>>>(key, emit, (uint32_t)n, (uint32_t)tiles,
-                                                                                         flag_words.get(), tile_cnt.get(), d_total,
-                                                                                         run_of_pos, sentinel);
+                                                                                         words, tile_cnt.get(), d_total,
+                                                                                         run_of_pos, sentinel, word_off);
         OL_CHECK_LAUNCH();
         return;
     }
