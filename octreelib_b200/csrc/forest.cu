@@ -918,7 +918,9 @@ __global__ void assign_epochs_kernel(uint32_t I, const uint32_t* __restrict__ ic
     iepoch[i] = out;
 }
 
-// recorded split node -> key under the NEW cell table (binary search of the packed cell key); ~0 if the cell is gone
+// recorded split node -> key under the NEW cell table (binary search of the packed cell key); ~0 if the cell is gone.
+// A node of a cell outside the key's range is dropped: below qmin, or with a field that spills into the next one (or past
+// bit 63), its packed key could equal that of a cell the forest holds.  The key is valid only if it unpacks to the node's q.
 __global__ void replay_keys_kernel(uint32_t n, const long long* __restrict__ q_in, const uint32_t* __restrict__ depth_in,
                                    const uint64_t* __restrict__ path_in, const uint64_t* __restrict__ cell_key, uint32_t C,
                                    KeyParams kp, uint64_t* __restrict__ keys, uint32_t* __restrict__ vals) {
@@ -928,13 +930,18 @@ __global__ void replay_keys_kernel(uint32_t n, const long long* __restrict__ q_i
     uint64_t packed = 0;
     bool ok = true;
     if (!kp.single_cell) {
+        long long q[3];
 #pragma unroll
         for (int a = 0; a < 3; ++a) {
-            const long long rel = q_in[(size_t)i * 3 + a] - kp.qmin[a];
+            q[a] = q_in[(size_t)i * 3 + a];
+            const long long rel = q[a] - kp.qmin[a];
             if (rel < 0) ok = false;
             const int s = kp.shift[a] - kp.pose_bits;
             if (ok && s < 64) packed |= ((uint64_t)rel) << s;
         }
+        long long back[3];
+        unpack_cell(kp, packed, back);
+        ok = ok && back[0] == q[0] && back[1] == q[1] && back[2] == q[2];
     }
     if (ok) {
         uint32_t lo = 0, hi = C;

@@ -54,6 +54,48 @@ def test_sort_all_equal_and_presorted():
     assert (gk == keys).all() and (gv == vals[::-1]).all()
 
 
+def _coherent_keys(n, dtype, begin, end, seed):
+    """keys as a LiDAR map gives them to the grid sort: 97 ascending runs over the whole key range [begin, end), each
+    with local noise and repeats; the bits outside the range are random"""
+    rng = np.random.default_rng(seed)
+    width, runs = end - begin, 97
+    i = np.arange(n, dtype=np.uint64)
+    run_len = (n + runs - 1) // runs
+    step = np.uint64(max((1 << width) // run_len, 1))
+    key = (i % np.uint64(run_len)) * step + rng.integers(0, 8 * int(step), size=n, dtype=np.uint64)
+    key += (i // np.uint64(run_len)) * np.uint64(0x9E3779B97F4A7C15)  # each run starts elsewhere (wraps mod 2^64)
+    rep = np.arange(3, n, 5)
+    key[rep] = key[rep - 1]  # repeated keys: stability matters
+    if width < 64:
+        key &= np.uint64((1 << width) - 1)
+    total = 8 * np.dtype(dtype).itemsize
+    outside = rng.integers(0, 1 << 64, size=n, dtype=np.uint64) & np.uint64(((1 << total) - 1) ^ (((1 << width) - 1) << begin))
+    return ((key << np.uint64(begin)) | outside).astype(dtype)
+
+
+@pytest.mark.parametrize("dtype,bits", [(np.uint32, (7, 29)), (np.uint32, (0, 23)), (np.uint32, (0, 32)),
+                                        (np.uint64, (0, 33)), (np.uint64, (0, 64))])
+def test_sort_pairs_at_the_grid_key_widths(dtype, bits):
+    """The grid sort runs on bits [fw, fw + key_bits): over 2^24 coherent keys the decoupled look-back spans > 4000 tiles.
+    Both onesweep tile shapes: 256 threads x 16 pairs (variant 0, the default) and 512 x 8 (variant 1)."""
+    from octreelib_b200 import _native as N
+    n = (1 << 24) + 5
+    keys = _coherent_keys(n, dtype, *bits, seed=bits[1])
+    vals = np.arange(n, dtype=np.uint32)
+    field = (keys.astype(np.uint64) >> np.uint64(bits[0]))
+    if bits[1] - bits[0] < 64:
+        field &= np.uint64((1 << (bits[1] - bits[0])) - 1)
+    order = np.argsort(field, kind="stable")
+    for variant in (0, 1):
+        N.lib().ol_debug_sort_variant(variant)
+        try:
+            gk, gv = sort_pairs(keys, vals, *bits)
+        finally:
+            N.lib().ol_debug_sort_variant(0)
+        assert (gv == vals[order]).all(), f"tile shape {variant}: values out of stable order"
+        assert (gk == keys[order]).all(), f"tile shape {variant}: keys out of order"
+
+
 @pytest.mark.parametrize("n", [4097, 250_000])
 def test_legacy_sort_path_agrees_with_onesweep(n):
     """radix_sort_pairs uses onesweep below 2^30 pairs and the three-kernel LSD sort above it; the
