@@ -42,7 +42,8 @@ typedef enum ol_status {
     OL_ERR_STATE = 8,       /* call not valid in the current state  -> RuntimeError */
     OL_ERR_POSE = 9,        /* unknown pose index                   -> KeyError */
     OL_ERR_INTERNAL = 10,   /* self-check failed (RANSAC verify)    -> AssertionError */
-    OL_ERR_CAPACITY = 11    /* exchange receive buffer too small    -> the host binding grows it and retries */
+    OL_ERR_CAPACITY = 11,   /* exchange receive buffer too small    -> the host binding grows it and retries */
+    OL_ERR_UNSUPPORTED = 12 /* result the grid cannot represent     -> NotImplementedError */
 } ol_status;
 
 typedef void *(*ol_alloc_fn)(void *user, size_t bytes);
@@ -196,6 +197,26 @@ int ol_forest_apply_mask(ol_forest *f);
  * points with mask 0 are removed. */
 int ol_forest_apply_pose_mask(ol_forest *f, const int32_t *pose_rank, int32_t pose_index, const uint8_t *mask_host,
                               int64_t n);
+
+/* ---- declarative leaf maps: Grid.map_leaf_points, grid.py:111-122 -> octree.py:114-123 ------------
+ * (octreelib_b200/leaf_maps.py: Centroid, Shrink, FirstPoints).  Every non-empty (pose, leaf) block of the listed poses
+ * (n_poses == 0: all poses) is mapped on the device, in float64, bit for bit like numpy on the block's points in
+ * ol_forest_export_points(order 0) order:
+ *   OL_MAP_CENTROID  the block becomes its mean, cloud.mean(axis=0) (sequential row sum / n);      param ignored
+ *   OL_MAP_SHRINK    every point p becomes c + param * (p - c), c the block's mean, no FMA;         param finite
+ *   OL_MAP_FIRST     the block keeps its first min(param, n) points (K7 compaction only);           param >= 0
+ * A result that is a subsequence of the block's own rows (a centroid equal to one of its points, a shrink that changes
+ * no point) keeps those rows, as the host path does with a callable.  Any other result replaces the block: its points
+ * are removed, the new rows are appended to the pose (one segment per pose, continuing the pose's point indices) and the
+ * grid is rebuilt with the same shape (scheme replay).  A new row outside the leaf it was computed from
+ * (lo <= p < lo + edge per axis, non-finite fails) returns OL_ERR_UNSUPPORTED before anything changes; an appended row
+ * that lands in another leaf after the rebuild returns OL_ERR_STATE.  rows_appended_host (NULL or [number of poses]
+ * int64) receives the rows appended to every pose index. */
+#define OL_MAP_CENTROID 0
+#define OL_MAP_SHRINK 1
+#define OL_MAP_FIRST 2
+int ol_forest_map_leaves(ol_forest *f, int32_t op, double param, const int32_t *pose_indices, int32_t n_poses,
+                         int64_t *rows_appended_host);
 
 /* Octree.subdivide_as / OctreeNode.subdivide_as (octree/octree.py:34-53, 222-227): copy the subdivision scheme of one
  * octree onto another.  ol_forest_export_shape lists the split nodes of a forest (cell coordinates q[n][3], depth, Morton

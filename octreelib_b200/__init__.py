@@ -13,7 +13,7 @@ import importlib
 import sys
 
 __version__ = "0.1.0"
-__all__ = ["install_as", "release_cached_memory", "grid", "octree", "octree_manager", "internal", "ransac", "criteria"]
+__all__ = ["install_as", "release_cached_memory", "grid", "octree", "octree_manager", "internal", "ransac", "criteria", "leaf_maps"]
 
 _SUBMODULES = ["internal", "internal.interfaces", "internal.point", "internal.typing", "internal.voxel", "octree",
                "octree.octree_base", "octree.octree", "octree_manager", "octree_manager.octree_manager", "ransac",
@@ -38,6 +38,6 @@ def release_cached_memory() -> int:
 
 
 def __getattr__(attr):
-    if attr in ("grid", "octree", "octree_manager", "internal", "ransac", "criteria"):
+    if attr in ("grid", "octree", "octree_manager", "internal", "ransac", "criteria", "leaf_maps"):
         return importlib.import_module(f"{__name__}.{attr}")
     raise AttributeError(attr)

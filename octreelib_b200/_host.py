@@ -11,6 +11,7 @@ import numpy as np
 from . import _views
 from .criteria import CountCriterion, GeometricCriterion, NotCountOnly, as_threshold, fold_count_criteria, fold_levels
 from .forest import Forest
+from .leaf_maps import Centroid, FirstPoints, Shrink
 
 __all__ = ["ForestHost"]
 
@@ -246,7 +247,33 @@ class ForestHost:
             self.forest.apply_pose_mask(p, mask)
 
     # ---- generic per-leaf callback (grid.py:111-122 -> octree_manager.py:68-83 -> octree.py:114-123) -----
+    _DEVICE_LEAF_MAPS = (Centroid, Shrink, FirstPoints)
+
     def map_leaf_points(self, function: Callable, pose_numbers: Optional[Sequence[int]] = None):
+        """`Centroid`, `Shrink` and `FirstPoints` (leaf_maps.py) run on the device (`ol_forest_map_leaves`) with the
+        result of the host path below; any other callable - subclasses of those included, which may redefine `__call__` -
+        takes the host path."""
+        if type(function) not in self._DEVICE_LEAF_MAPS:
+            self._map_leaf_points_on_host(function, pose_numbers)
+            return
+        if self.empty:
+            return
+        if pose_numbers is None:
+            idx = None
+        else:
+            # unknown numbers are ignored like on the host path; a pose listed twice is mapped once
+            idx = list(dict.fromkeys(self.pose_index[p] for p in pose_numbers if p in self.pose_index))
+            if not idx:
+                return
+        rows = np.zeros(max(len(self.pose_numbers), 1), dtype=np.int64)
+        try:
+            self.forest.map_leaves(function.op, function.param, idx, rows)
+        finally:  # (a failed post-rebuild check raises with the rows appended, like the host path)
+            for p in np.flatnonzero(rows[:len(self.pose_inserted)]):
+                self.pose_inserted[p] += int(rows[p])
+            self._counts_cache = None
+
+    def _map_leaf_points_on_host(self, function: Callable, pose_numbers: Optional[Sequence[int]] = None):
         """Host-callback compatibility path (SURVEY 8(f) rank 1): every non-empty (pose, leaf) block is copied to the
         host, handed to the opaque Python `function`, and the result replaces the block's points
         (grid.py:111-122 -> octree_manager.py:68-83 -> octree.py:114-123).  Like the reference, empty leaves are skipped

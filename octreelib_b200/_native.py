@@ -20,6 +20,8 @@ OL_MAX_DEPTH = 21
 RANSAC_FLAG_NO_TMA, RANSAC_FLAG_EXACT_ONLY, RANSAC_FLAG_VERIFY, RANSAC_FLAG_STATS = 1, 2, 4, 8
 OL_ERR_INTERNAL = 10
 OL_ERR_CAPACITY = 11
+OL_ERR_UNSUPPORTED = 12
+OL_MAP_CENTROID, OL_MAP_SHRINK, OL_MAP_FIRST = 0, 1, 2
 
 ALLOC_FN = C.CFUNCTYPE(C.c_void_p, C.c_void_p, C.c_size_t)
 FREE_FN = C.CFUNCTYPE(None, C.c_void_p, C.c_void_p)
@@ -88,6 +90,7 @@ SIGNATURES = {
     "ol_forest_pose_point_counts": (C.c_int, [_p, _p]),
     "ol_forest_apply_mask": (C.c_int, [_p]),
     "ol_forest_apply_pose_mask": (C.c_int, [_p, _p, _i32, _p, _i64]),
+    "ol_forest_map_leaves": (C.c_int, [_p, _i32, _f64, _p, _i32, _p]),
     "ol_forest_profile": (C.c_int, [_p, _i32]),
     "ol_forest_profile_read": (C.c_int, [_p, C.c_char_p, _i64, C.POINTER(_i64)]),
     "ol_launch_count": (_u64, []),
@@ -162,6 +165,7 @@ _EXC = {
     OL_ERR_POSE: KeyError,
     OL_ERR_INTERNAL: AssertionError,
     OL_ERR_CAPACITY: ExchangeCapacityError,
+    OL_ERR_UNSUPPORTED: NotImplementedError,
 }
 
 

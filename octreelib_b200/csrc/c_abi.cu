@@ -342,6 +342,16 @@ int ol_forest_apply_pose_mask(ol_forest* f, const int32_t* pose_rank, int32_t po
     OL_API_END
 }
 
+int ol_forest_map_leaves(ol_forest* f, int32_t op, double param, const int32_t* pose_indices, int32_t n_poses,
+                         int64_t* rows_appended_host) {
+    OL_NEED(f);
+    OL_API_BEGIN
+    OL_REQUIRE(n_poses >= 0 && (n_poses == 0 || pose_indices), OL_ERR_INVALID, "bad pose list");
+    ForestScope scope(f->impl);
+    f->impl.map_leaves(op, param, pose_indices, n_poses, rows_appended_host);
+    OL_API_END
+}
+
 int ol_forest_profile(ol_forest* f, int32_t enable) {
     OL_NEED(f);
     OL_API_BEGIN

@@ -73,6 +73,8 @@ enum DevErr : uint32_t {
     DEVERR_DEPTH_CAP = 8u,      // a node still exceeds the criterion at the maximum depth
     DEVERR_SAMPLE_OOB = 16u,    // RANSAC sample index fell outside its block (clamped)
     DEVERR_FILTER_BOUND = 32u,  // RANSAC verify mode: an exact count left its pre-filter interval
+    DEVERR_LEAF_MAP = 64u,      // a leaf map produced a row outside the leaf it was computed from (leaf_maps.cuh)
+    DEVERR_LEAF_MOVED = 128u,   // an appended leaf-map row landed in another leaf after the rebuild
 };
 
 // ---------------------------------------------------------------------------------------------

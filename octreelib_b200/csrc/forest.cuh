@@ -271,6 +271,8 @@ struct Forest {
     void materialize_snapshot();
     void drop_snapshot();
     void apply_pose_mask(const int32_t* pose_rank, int pose, const uint8_t* mask_host, int64_t n);
+    // declarative leaf maps (leaf_maps.cuh, ol_forest_map_leaves); rows_appended: NULL or [n_poses]
+    void map_leaves(int op, double param, const int32_t* poses, int n_poses_listed, int64_t* rows_appended);
     void pose_counts(int64_t* out_host);
     void stats(ol_forest_stats* s, bool light = false);
     std::string profile_report();  // "name count total_ms" per line; clears the records

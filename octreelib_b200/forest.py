@@ -385,6 +385,20 @@ class Forest:
             N.check(self._lib.ol_forest_apply_pose_mask(self._h, None, int(pose_index), _ptr(m), len(m)))
         self.version += 1
 
+    def map_leaves(self, op: int, param: float, pose_indices: Optional[Sequence[int]] = None,
+                   rows: Optional[np.ndarray] = None) -> np.ndarray:
+        """Declarative leaf map of every non-empty block of the listed poses (all: None) on the device
+        (`ol_forest_map_leaves`, op = N.OL_MAP_*).  Returns the rows appended to every pose index; `rows` (int64, one entry
+        per pose at least) receives them even when the call raises after appending."""
+        arr, n = _i32_array(pose_indices)
+        if rows is None:
+            rows = np.zeros(max(self._n_poses_native + len(self._batch), 1), dtype=np.int64)
+        assert rows.dtype == np.int64 and rows.flags.c_contiguous and len(rows) >= self._n_poses_native + len(self._batch)
+        with self._scope():
+            N.check(self._lib.ol_forest_map_leaves(self._h, int(op), float(param), _ptr(arr), n, _ptr(rows)))
+        self.version += 1
+        return rows
+
     # ---- measurement ---------------------------------------------------------------------------
     def profile(self, enable: bool = True):
         with self._scope():

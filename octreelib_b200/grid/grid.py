@@ -65,8 +65,9 @@ class Grid(GridBase):
 
     # ---- grid.py:111-122 ------------------------------------------------------------------------
     def map_leaf_points(self, function: Callable[[PointCloud], PointCloud], pose_numbers: Optional[List[int]] = None):
-        """Host-callback compatibility path: see ForestHost.map_leaf_points (the function must return a selection of
-        the leaf's own points).  The data-parallel equivalents are `filter` and `map_leaf_points_cuda_ransac`."""
+        """`Centroid()`, `Shrink(factor)` and `FirstPoints(k)` (octreelib_b200.leaf_maps) run on the GPU; any other
+        callable takes the host-callback compatibility path: see ForestHost.map_leaf_points (the result must lie inside
+        the leaf it was computed from).  Other data-parallel equivalents are `filter` and `map_leaf_points_cuda_ransac`."""
         self._host.map_leaf_points(function, pose_numbers)
 
     # ---- grid.py:124-215 ------------------------------------------------------------------------
