@@ -405,8 +405,6 @@ int ol_sort_pairs_u32(void *stream, uint32_t *keys_dev, uint32_t *vals_dev, int6
                       int32_t end_bit, ol_alloc_fn alloc, ol_free_fn free_fn, void *alloc_user);
 /* test hook: 1 = use the three-kernel LSD sort instead of onesweep (both must give identical results) */
 int ol_debug_force_legacy_sort(int32_t on);
-/* test / tuning hook: tile shape of the onesweep pass kernel (0 = default: 256 threads x 16 pairs, 1 = 512 x 8; measured A/B in profiles/) */
-int ol_debug_sort_variant(int32_t variant);
 /* exclusive prefix sum, in place allowed; total written to *total_host if non-NULL (synchronises) */
 int ol_exclusive_scan_u32(void *stream, const uint32_t *in_dev, uint32_t *out_dev, int64_t n, uint64_t *total_host,
                           ol_alloc_fn alloc, ol_free_fn free_fn, void *alloc_user);

@@ -124,7 +124,6 @@ SIGNATURES = {
     "ol_sort_pairs_u64": (C.c_int, [_p, _p, _p, _i64, _i32, _i32, ALLOC_FN, FREE_FN, _p]),
     "ol_sort_pairs_u32": (C.c_int, [_p, _p, _p, _i64, _i32, _i32, ALLOC_FN, FREE_FN, _p]),
     "ol_debug_force_legacy_sort": (C.c_int, [_i32]),
-    "ol_debug_sort_variant": (C.c_int, [_i32]),
     "ol_exclusive_scan_u32": (C.c_int, [_p, _p, _p, _i64, C.POINTER(_u64), ALLOC_FN, FREE_FN, _p]),
     "ol_host_floor_divide": (_f64, [_f64, _f64]),
     "ol_host_point_key": (C.c_int, [_f64, C.POINTER(_f64 * 3), _i32, _i32, C.POINTER(_f64 * 3),

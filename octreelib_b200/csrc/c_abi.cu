@@ -50,7 +50,6 @@ MailResult mail_wait(const Mail& m, cudaStream_t stream) {
     r.aux = (uint32_t)m.slot[3];
     return r;
 }
-int g_os_variant = 0;
 static thread_local std::string g_last_error;
 void set_last_error(int code, const std::string& msg) { g_last_error = "[ol_status " + std::to_string(code) + "] " + msg; }
 }  // namespace ol
@@ -618,11 +617,6 @@ int ol_measure_fma_peak(void* stream, double* out_fp64_tflops, double* out_fp32_
 }
 
 // ---- primitives ---------------------------------------------------------------------------------
-int ol_debug_sort_variant(int32_t variant) {
-    ol::g_os_variant = variant;
-    return OL_OK;
-}
-
 int ol_debug_force_legacy_sort(int32_t on) {
     ol::g_force_legacy_sort = on != 0;
     return OL_OK;

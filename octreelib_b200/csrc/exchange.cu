@@ -733,8 +733,7 @@ void Exchange::run(Forest& f, const double* const* clouds, const int64_t* sizes,
     // Keys, sort and cell table are enqueued right behind the scatter (the cell-coordinate range came with the plan, so
     // nothing has to be read back first): the GPU keeps working while the host language returns from this call and
     // prepares the next one; the number of cells is picked up from the mailbox by that next call.
-    static const bool no_eager = getenv("OL_NO_PREFETCH") != nullptr;
-    if (!no_eager) f.build_enqueue();
+    f.build_enqueue();
 }
 
 }  // namespace ol

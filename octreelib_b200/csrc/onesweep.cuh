@@ -23,34 +23,18 @@ constexpr int OS_ITEMS = 16;
 constexpr int OS_TILE = OS_THREADS * OS_ITEMS;
 constexpr int OS_WARPS = OS_THREADS / 32;
 constexpr int OS_MAX_PASSES = 8;
-#ifndef OS_LOOKBACK
-#define OS_LOOKBACK 4  // measured on the 100 M-pair pass: 1 -> 0.68 ms, 4 -> 0.617, 8 -> 0.627, 16 -> 0.653
-#endif
+constexpr int OS_LOOKBACK = 4;  // measured on the 100 M-pair pass: 1 -> 0.68 ms, 4 -> 0.617, 8 -> 0.627, 16 -> 0.653
 constexpr uint32_t OS_FLAG_AGG = 1u << 30;
 constexpr uint32_t OS_FLAG_INC = 2u << 30;
 constexpr uint32_t OS_VAL_MASK = (1u << 30) - 1u;
 
-// Lanes whose digit equals this lane's digit.  MATCH.ANY is microcoded - its cost grows with the number of
-// distinct values in the warp (~28 for random 8-bit digits: > 50 % of a pass on random keys); the alternative
-// (-DOS_MATCH_BALLOT) builds the peer mask from one ballot per digit bit, which is faster on random keys but
-// slower on coherent ones.  Invalid lanes only match each other.
-__device__ __forceinline__ uint32_t os_match_digit(uint32_t d, int nbits, bool valid) {
-#ifndef OS_MATCH_BALLOT
-    // spatially coherent keys (LiDAR scan order) put few distinct digits in a warp, where MATCH.ANY is the
-    // cheaper instruction: measured 0.81 ms vs 1.2 ms per 100 M-pair pass on the bench workload
+// Lanes whose digit equals this lane's digit; invalid lanes only match each other.  MATCH.ANY is microcoded - its
+// cost grows with the number of distinct values in the warp (~28 for random 8-bit digits: > 50 % of a pass on random
+// keys).  A peer mask built from one ballot per digit bit is faster on random keys, but spatially coherent keys (LiDAR
+// scan order) put few distinct digits in a warp, where MATCH.ANY is the cheaper instruction: measured 0.81 ms vs
+// 1.2 ms per 100 M-pair pass on the bench workload.
+__device__ __forceinline__ uint32_t os_match_digit(uint32_t d, bool valid) {
     return __match_any_sync(0xffffffffu, valid ? d : 0xffffffffu);
-#endif
-    uint32_t peers = __ballot_sync(0xffffffffu, valid);
-    if (!valid) peers = ~peers;
-#pragma unroll
-    for (int b = 0; b < 8; ++b) {
-        if (b < nbits) {  // warp-uniform
-            const bool bit = (d >> b) & 1u;
-            const uint32_t v = __ballot_sync(0xffffffffu, bit);
-            peers &= bit ? v : ~v;
-        }
-    }
-    return peers;
 }
 
 struct OsPlan {
@@ -169,14 +153,12 @@ __device__ __forceinline__ void os_st_status(uint32_t* p, uint32_t v) {
     asm volatile("st.relaxed.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
 }
 
-template <typename KeyT, int OS_THREADS, int OS_ITEMS, int MIN_BLOCKS>
-__global__ void __launch_bounds__(OS_THREADS, MIN_BLOCKS) os_pass_kernel(const KeyT* __restrict__ keys_in, const uint32_t* __restrict__ vals_in,
-                                                             KeyT* __restrict__ keys_out, uint32_t* __restrict__ vals_out,
-                                                             const uint32_t* __restrict__ gbase /*[256] exclusive digit offsets*/,
-                                                             uint32_t* __restrict__ status /*[tiles][256]*/,
-                                                             uint32_t* __restrict__ tile_counter, uint32_t n, int shift, int nbits) {
-    constexpr int OS_TILE = OS_THREADS * OS_ITEMS;
-    constexpr int OS_WARPS = OS_THREADS / 32;
+template <typename KeyT>
+__global__ void __launch_bounds__(OS_THREADS, 3) os_pass_kernel(const KeyT* __restrict__ keys_in, const uint32_t* __restrict__ vals_in,
+                                                                KeyT* __restrict__ keys_out, uint32_t* __restrict__ vals_out,
+                                                                const uint32_t* __restrict__ gbase /*[256] exclusive digit offsets*/,
+                                                                uint32_t* __restrict__ status /*[tiles][256]*/,
+                                                                uint32_t* __restrict__ tile_counter, uint32_t n, int shift, int nbits) {
     extern __shared__ __align__(16) unsigned char os_smem[];
     KeyT* s_keys = reinterpret_cast<KeyT*>(os_smem);                                // [OS_TILE]
     uint32_t* s_vals = reinterpret_cast<uint32_t*>(os_smem + sizeof(KeyT) * OS_TILE);  // [OS_TILE]
@@ -228,7 +210,7 @@ __global__ void __launch_bounds__(OS_THREADS, MIN_BLOCKS) os_pass_kernel(const K
         const uint32_t i = wbase + j * 32 + lane;
         const bool valid = i < n;
         const uint32_t d = (uint32_t)(k[j] >> shift) & mask;
-        const uint32_t peers = os_match_digit(d, nbits, valid);
+        const uint32_t peers = os_match_digit(d, valid);
         const int leader = __ffs(peers) - 1;
         uint32_t old = 0;
         if (valid && lane == leader) {
@@ -330,27 +312,22 @@ __global__ void __launch_bounds__(OS_THREADS, MIN_BLOCKS) os_pass_kernel(const K
     }
 }
 
-template <typename KeyT, int THREADS, int ITEMS>
+template <typename KeyT>
 inline size_t os_pass_smem() {
-    return sizeof(KeyT) * THREADS * ITEMS + 4 * THREADS * ITEMS + 4 * ((THREADS / 32) * 256 + 256 + 256) + 4 * THREADS * ITEMS;
+    return sizeof(KeyT) * OS_TILE + 4 * OS_TILE + 4 * (OS_WARPS * 256 + 256 + 256) + 4 * OS_TILE;
 }
 
-// tile shapes selectable at run time (ol_debug_sort_variant): A/B measurements inside one process
-extern int g_os_variant;
-
-template <typename KeyT, int THREADS, int ITEMS, int MIN_BLOCKS>
+template <typename KeyT>
 inline void os_launch_pass(Ctx& c, const KeyT* kin, const uint32_t* vin, KeyT* kout, uint32_t* vout, const uint32_t* gbase,
                            uint32_t* status, uint32_t* counter, uint32_t n, int shift, int nbits) {
     static bool attr_set = false;
-    const size_t smem = os_pass_smem<KeyT, THREADS, ITEMS>();
+    const size_t smem = os_pass_smem<KeyT>();
     if (!attr_set) {
-        OL_CUDA(cudaFuncSetAttribute(os_pass_kernel<KeyT, THREADS, ITEMS, MIN_BLOCKS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)smem));
+        OL_CUDA(cudaFuncSetAttribute(os_pass_kernel<KeyT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         attr_set = true;
     }
-    const uint32_t tiles = (n + THREADS * ITEMS - 1) / (THREADS * ITEMS);
-    os_pass_kernel<KeyT, THREADS, ITEMS, MIN_BLOCKS><<<tiles, THREADS, smem, c.stream>>>(kin, vin, kout, vout, gbase, status, counter, n,
-                                                                                        shift, nbits);
+    const uint32_t tiles = (n + OS_TILE - 1) / OS_TILE;
+    os_pass_kernel<KeyT><<<tiles, OS_THREADS, smem, c.stream>>>(kin, vin, kout, vout, gbase, status, counter, n, shift, nbits);
     OL_CHECK_LAUNCH();
 }
 
@@ -362,10 +339,9 @@ inline int onesweep_sort_pairs(Ctx& c, KeyT* keys0, KeyT* keys1, uint32_t* vals0
     const OsPlan plan = os_make_plan(begin_bit, end_bit);
     OL_REQUIRE(plan.passes <= OS_MAX_PASSES, OL_ERR_INVALID, "onesweep: too many digit passes");
     const uint32_t tiles = (uint32_t)((n + OS_TILE - 1) / OS_TILE);
-    const uint32_t max_tiles = tiles;  // both tile shapes hold 4096 pairs
     // [passes][256] histograms | [passes] tile counters | [tiles][256] status words (re-zeroed per pass)
     // (one status array PER PASS, all of them zeroed by one memset: a memset per pass was a 2 us operation plus a 2 us bubble)
-    const size_t status_per_pass = (size_t)max_tiles * 256;
+    const size_t status_per_pass = (size_t)tiles * 256;
     DevBuf<uint32_t> ghist(c, (size_t)plan.passes * 256 + OS_MAX_PASSES), status(c, status_per_pass * (size_t)plan.passes);
     ghist.zero();
     status.zero();
@@ -390,10 +366,7 @@ inline int onesweep_sort_pairs(Ctx& c, KeyT* keys0, KeyT* keys1, uint32_t* vals0
         ProfScope ps(c, sname, (double)n);
         const uint32_t* gb = ghist.get() + (size_t)p * 256;
         uint32_t* ctr = ghist.get() + (size_t)plan.passes * 256 + p;
-        switch (g_os_variant) {
-            case 1: os_launch_pass<KeyT, 512, 8, 2>(c, kin, vin, kout, vout, gb, status_p, ctr, (uint32_t)n, plan.bit[p], plan.nbits[p]); break;
-            default: os_launch_pass<KeyT, 256, 16, 3>(c, kin, vin, kout, vout, gb, status_p, ctr, (uint32_t)n, plan.bit[p], plan.nbits[p]); break;
-        }
+        os_launch_pass<KeyT>(c, kin, vin, kout, vout, gb, status_p, ctr, (uint32_t)n, plan.bit[p], plan.nbits[p]);
         cur ^= 1;
     }
     return cur;

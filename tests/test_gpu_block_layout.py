@@ -1,19 +1,20 @@
 """The sort-free RANSAC batch layout (leaf spans from the run index of the block build, work list written by the ranking)
-and the block of every position derived on demand must give what the sorted layout gives (OL_RANSAC_SORTED_LAYOUT=1, in
-a subprocess) on the shapes where they are easiest to get wrong.  Run as a script, this file prints the digest of one
-case."""
+and the block of every position derived on demand must give what the sorted layout gives, on the shapes where they are
+easiest to get wrong.  The layout follows the pose ranks: dense ranks below REFSTART_MAX_RANKS (2048) take the sort-free
+one; the same ranks shifted past it by a whole number of batches take the sorted one.  Batches are the groups
+rank // poses_per_batch and every start index is relative to its batch, so the shift changes nothing in the result."""
 import hashlib
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 
-HERE = os.path.dirname(os.path.abspath(__file__))
-sys.path.insert(0, os.path.dirname(HERE))
-
 K = 6
+REFSTART_MAX_RANKS = 2048
+
+
+def _rank_offset(poses_per_batch):
+    """the smallest multiple of poses_per_batch that is at least REFSTART_MAX_RANKS: 2048 for 2, 2049 for 3"""
+    return -(-REFSTART_MAX_RANKS // poses_per_batch) * poses_per_batch
 
 
 def _blob(rng, n, lo, hi):
@@ -37,7 +38,7 @@ def _clouds(case):
     raise KeyError(case)
 
 
-def digest(case):
+def digest(case, shifted):
     from octreelib_b200.criteria import MaxPoints, MinPoints
     from octreelib_b200.grid import Grid, GridConfig
     from octreelib_b200.ransac import CudaRansac
@@ -52,13 +53,17 @@ def digest(case):
     pose_rank = [int(x) for x in host.pose_numbers]
     h = hashlib.sha256()
 
+    def ranks(ppb):
+        off = _rank_offset(ppb) if shifted else 0
+        return [r + off for r in pose_rank]
+
     def add(*arrays):
         for a in arrays:
             h.update(np.ascontiguousarray(a).tobytes())
 
     np.random.seed(5)
     table = CudaRansac(threshold=0.02, hypotheses_number=256, initial_points_number=K).random_hypotheses
-    forest.ransac(table, 0.02, pose_rank, 3, apply=False)
+    forest.ransac(table, 0.02, ranks(3), 3, apply=False)
     res = forest.export_ransac()
     add(*(res[k] for k in ("pose", "leaf", "size", "plane", "best", "best_count")))
     scored = forest.export_ransac(scored_only=True)
@@ -69,7 +74,8 @@ def digest(case):
     pts = forest.export_points(-1, order=1, want_mask=True)  # block of every position, same block table as the fit
     add(pts["idx"], pts["xyz"])
     np.random.seed(7)
-    grid.map_leaf_points_cuda_ransac(poses_per_batch=2, threshold=0.02, hypotheses_number=256, initial_points_number=K)
+    table = CudaRansac(threshold=0.02, hypotheses_number=256, initial_points_number=K).random_hypotheses
+    forest.ransac(table, 0.02, ranks(2), 2, apply=True)  # what map_leaf_points_cuda_ransac does, at the chosen ranks
     res = forest.export_ransac(scored_only=True)
     add(*(res[k] for k in ("pose", "leaf", "size", "plane", "best", "best_count")))
     for p in numbers[:3]:
@@ -86,12 +92,4 @@ def digest(case):
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", ["one_block", "straddle", "all_small", "ranks"])
 def test_fast_layout_matches_sorted_layout(case):
-    env = dict(os.environ, OL_RANSAC_SORTED_LAYOUT="1")
-    out = subprocess.run([sys.executable, os.path.abspath(__file__), case], env=env, capture_output=True, text=True, timeout=600)
-    assert out.returncode == 0, out.stderr[-2000:]
-    sorted_digest = [l for l in out.stdout.splitlines() if l.startswith("DIGEST ")][-1].split()[1]
-    assert digest(case) == sorted_digest
-
-
-if __name__ == "__main__":
-    print("DIGEST", digest(sys.argv[1]))
+    assert digest(case, shifted=False) == digest(case, shifted=True)

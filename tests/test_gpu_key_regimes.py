@@ -14,10 +14,12 @@ import numpy as np
 import pytest
 
 from gpu_util import compare_grid_with_oracle
-from octreelib_b200.criteria import MaxExtent, MaxPoints, MinPoints, extent
+from octreelib_b200.criteria import MaxExtent, MaxPoints, MinPoints, Planar, extent
 from octreelib_b200.grid import Grid, GridConfig
+from octreelib_b200.leaf_maps import Centroid, FirstPoints, Shrink
 from oracle import ransac as oransac
 from oracle.structure import OracleGrid
+from test_gpu_geometric_criteria import _assert_clear_of_threshold
 
 pytestmark = pytest.mark.gpu
 U = 2.0 ** -53
@@ -81,6 +83,31 @@ def _build(edge, clouds):
         grid.insert_points(p, c)
         og.insert_points(p, c)
     return grid, og
+
+
+# subclasses of the declarative leaf maps take the host path: the object's own __call__ once per (pose, leaf) block
+class _HostCentroid(Centroid):
+    pass
+
+
+class _HostShrink(Shrink):
+    pass
+
+
+class _HostFirstPoints(FirstPoints):
+    pass
+
+
+def _same_leaves(ga, gb, poses):
+    for p in poses:
+        va, vb = ga.get_leaf_points(p), gb.get_leaf_points(p)
+        assert len(va) == len(vb)
+        for x, y in zip(va, vb):
+            assert (np.asarray(x.corner_min) == np.asarray(y.corner_min)).all() and x.edge_length == y.edge_length
+            assert (np.asarray(x.get_points()) == np.asarray(y.get_points())).all()
+        ea, eb = (g._host.forest.export_points(g._host.pose_index[p], order=0) for g in (ga, gb))
+        assert (ea["xyz"] == eb["xyz"]).all() and (ea["idx"] == eb["idx"]).all()
+        assert [ga.n_leaves(p), ga.n_points(p), ga.n_nodes(p)] == [gb.n_leaves(p), gb.n_points(p), gb.n_nodes(p)]
 
 
 def _both(grid, og, call, *args):
@@ -153,6 +180,25 @@ def test_regime_matches_the_oracle(key_bits):
     assert grid._host.forest.stats()["max_depth_reached"] > 10
     compare_grid_with_oracle(grid, og, [0, 1, 2, 3])
     _check_leaf_statistics(grid, og, [0, 1, 2, 3])
+    # 7. fresh builds of the first two poses (the key of this regime, no late pose to widen it): a geometric filter against
+    # the oracle, then the declarative leaf maps against the host path.  The maps replace the rows of pose 1 only: rows
+    # appended to the last pose keep the pose segments in order, so the rebuild keeps the key of the regime (an
+    # out-of-order segment would add a pose bit, which does not fit next to 64 cell bits)
+    first = {p: clouds[p] for p in (0, 1)}
+    grid, og = _build(edge, first)
+    _both(grid, og, "subdivide", [MaxPoints(40)])
+    assert grid._host.forest.stats()["key_bits"] == key_bits
+    planar = Planar(0.05 * edge)
+    _assert_clear_of_threshold([leaf.points for p in first for leaf in og.get_leaf_points(p)], planar.value, 3)
+    _both(grid, og, "filter", [planar])
+    compare_grid_with_oracle(grid, og, [0, 1])
+    for obj, on_host in ((Centroid(), _HostCentroid()), (Shrink(0.5), _HostShrink(0.5)), (FirstPoints(2), _HostFirstPoints(2))):
+        ga, gb = _build(edge, first)[0], _build(edge, first)[0]
+        for g, fn in ((ga, obj), (gb, on_host)):
+            g.subdivide([MaxPoints(40)])
+            g.filter([planar])
+            g.map_leaf_points(fn, [1])
+        _same_leaves(ga, gb, [0, 1])
 
 
 def test_more_than_64_key_bits_is_refused_and_leaves_no_error_behind():

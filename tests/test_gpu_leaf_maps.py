@@ -1,15 +1,12 @@
 """GPU: declarative leaf maps of `map_leaf_points` (Centroid, Shrink, FirstPoints; csrc/leaf_maps.cuh) against the
 reference fixture and against the host path, which calls the equivalent plain function once per (pose, leaf) block.
 Every comparison is bit for bit: points, leaf corners and edges, counters, and the point indices of export_points."""
-import os
-import subprocess
-import sys
+import hashlib
 
 import numpy as np
 import pytest
 
 from conftest import golden
-from leaf_map_digest import clustered_clouds, digest
 from octreelib_b200.criteria import MaxExtent, MaxPoints, MinPoints
 from octreelib_b200.grid import Grid, GridConfig
 from octreelib_b200.leaf_maps import Centroid, FirstPoints, Shrink
@@ -17,10 +14,19 @@ from test_gpu_key_regimes import REGIMES, box_cells, cluster, expected_key_bits
 from test_gpu_map_leaf_points import _check
 
 pytestmark = pytest.mark.gpu
-HERE = os.path.dirname(os.path.abspath(__file__))
 
 OBJECTS = [Centroid(), Shrink(0.5), Shrink(0.0), Shrink(0.9), FirstPoints(0), FirstPoints(1), FirstPoints(3),
            FirstPoints(1 << 40)]
+
+
+def clustered_clouds(seed, n_poses=3, n=1500):
+    rng = np.random.default_rng(seed)
+    out = {}
+    for p in range(n_poses):
+        centres = rng.uniform(-10, 14, (6, 3))
+        pts = np.vstack([c + rng.normal(0, rng.uniform(0.2, 1.5), (n // 6, 3)) for c in centres])
+        out[p] = np.vstack([pts, rng.uniform(-12, 16, (n // 5, 3))])
+    return out
 
 
 def plain(obj):
@@ -291,11 +297,20 @@ def test_no_per_block_python(monkeypatch):
         assert grid.n_points(1) > 0 and mp.n_points(1) > 0 and tree.n_points > 0
 
 
-# ---- 7. debug switches ----------------------------------------------------------------------------------------------
-def test_debug_switches_do_not_change_results():
-    ref = digest()
-    env = dict(os.environ, OL_NO_PREFETCH="1", OL_NO_EMBED="1", OL_RUNS_ONE_PASS="1")
-    out = subprocess.run([sys.executable, os.path.join(HERE, "leaf_map_digest.py")], env=env, capture_output=True, text=True,
-                         timeout=600)
-    assert out.returncode == 0, out.stderr[-2000:]
-    assert [l for l in out.stdout.splitlines() if l.startswith("DIGEST ")][-1].split()[1] == ref
+# ---- 7. repeatability -----------------------------------------------------------------------------------------------
+def _digest():
+    """digest of a grid after every declarative leaf map"""
+    h = hashlib.sha256()
+    for obj, poses in ((Shrink(0.5), None), (Centroid(), [2, 0]), (FirstPoints(2), None)):
+        grid = _grid(clustered_clouds(11), 4.0, [MaxPoints(25)])
+        grid.map_leaf_points(obj, poses)
+        for p in range(3):
+            e = grid._host.forest.export_points(grid._host.pose_index[p], order=0)
+            h.update(np.ascontiguousarray(e["xyz"]).tobytes())
+            h.update(np.ascontiguousarray(e["idx"]).tobytes())
+            h.update(np.array([grid.n_leaves(p), grid.n_points(p), grid.n_nodes(p)], dtype=np.int64).tobytes())
+    return h.hexdigest()
+
+
+def test_leaf_maps_are_bit_identical_across_runs():
+    assert _digest() == _digest()

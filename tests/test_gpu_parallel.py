@@ -77,7 +77,8 @@ def test_emulated_slab_ranks_reproduce_the_single_gpu_batch_layout():
     """Three 'ranks' with slab ownership, processed one after the other: with `pose_start` from the gathered pose sizes
     every rank's RANSAC uses the reference's batch-global block starts, so planes / winners / masks are bit-identical to
     the single-GPU grid at poses_per_batch = 2 - and the rank-major concatenation of the plane tables, sorted stably by
-    pose, is the single-GPU table row for row."""
+    pose, is the single-GPU table row for row.  The emulated ranks run twice: with the dense pose ranks (sort-free batch
+    layout) and with the ranks shifted by 2048, a whole number of batches of at least REFSTART_MAX_RANKS (sorted layout)."""
     from octreelib_b200.parallel import pose_starts
     from octreelib_b200.ransac import CudaRansac
 
@@ -110,21 +111,22 @@ def test_emulated_slab_ranks_reproduce_the_single_gpu_batch_layout():
         sizes[r] = f.pose_point_counts(P)
         forests.append(f)
     assert (sizes.sum(axis=0) == [len(clouds[p]) for p in range(P)]).all()
-    rows = []
-    leaf_base = 0
-    for r, f in enumerate(forests):
-        f.ransac(table, 0.02, list(range(P)), ppb, apply=False, pose_start=pose_starts(sizes, r, ppb))
-        got = f.export_ransac(scored_only=True)
-        lv = f.export_leaves()
-        for i in range(len(got["best"])):
-            rows.append((int(got["pose"][i]), r, i, tuple(lv["corner"][got["leaf"][i]]), float(lv["edge"][got["leaf"][i]]),
-                         int(got["best"][i]), int(got["best_count"][i]), got["plane"][i].tobytes()))
-        leaf_base += len(lv["edge"])
-    rows.sort(key=lambda t: (t[0], t[1], t[2]))  # stable by pose over the rank-major concatenation
-    assert len(rows) == len(want["best"])
-    for i, row in enumerate(rows):
-        assert row[0] == want["pose"][i] and row[3] == tuple(want_leaves["corner"][want["leaf"][i]])
-        assert row[5] == want["best"][i] and row[6] == want["best_count"][i] and row[7] == want["plane"][i].tobytes()
+    for rank_offset in (0, 2048):
+        rows = []
+        leaf_base = 0
+        for r, f in enumerate(forests):
+            f.ransac(table, 0.02, [p + rank_offset for p in range(P)], ppb, apply=False, pose_start=pose_starts(sizes, r, ppb))
+            got = f.export_ransac(scored_only=True)
+            lv = f.export_leaves()
+            for i in range(len(got["best"])):
+                rows.append((int(got["pose"][i]), r, i, tuple(lv["corner"][got["leaf"][i]]), float(lv["edge"][got["leaf"][i]]),
+                             int(got["best"][i]), int(got["best_count"][i]), got["plane"][i].tobytes()))
+            leaf_base += len(lv["edge"])
+        rows.sort(key=lambda t: (t[0], t[1], t[2]))  # stable by pose over the rank-major concatenation
+        assert len(rows) == len(want["best"]), rank_offset
+        for i, row in enumerate(rows):
+            assert row[0] == want["pose"][i] and row[3] == tuple(want_leaves["corner"][want["leaf"][i]]), rank_offset
+            assert row[5] == want["best"][i] and row[6] == want["best_count"][i] and row[7] == want["plane"][i].tobytes(), rank_offset
 
 
 def test_partition_by_owner_matches_host_rule():

@@ -75,10 +75,8 @@ def _coherent_keys(n, dtype, begin, end, seed):
 
 @pytest.mark.parametrize("dtype,bits", [(np.uint32, (7, 29)), (np.uint32, (0, 23)), (np.uint32, (0, 32)),
                                         (np.uint64, (0, 33)), (np.uint64, (0, 64))])
-def test_sort_pairs_at_the_grid_key_widths(dtype, bits):
-    """The grid sort runs on bits [fw, fw + key_bits): over 2^24 coherent keys the decoupled look-back spans > 4000 tiles.
-    Both onesweep tile shapes: 256 threads x 16 pairs (variant 0, the default) and 512 x 8 (variant 1)."""
-    from octreelib_b200 import _native as N
+def test_onesweep_sort_at_the_grid_key_widths(dtype, bits):
+    """The grid sort runs on bits [fw, fw + key_bits): over 2^24 coherent keys the decoupled look-back spans > 4000 tiles."""
     n = (1 << 24) + 5
     keys = _coherent_keys(n, dtype, *bits, seed=bits[1])
     vals = np.arange(n, dtype=np.uint32)
@@ -86,14 +84,9 @@ def test_sort_pairs_at_the_grid_key_widths(dtype, bits):
     if bits[1] - bits[0] < 64:
         field &= np.uint64((1 << (bits[1] - bits[0])) - 1)
     order = np.argsort(field, kind="stable")
-    for variant in (0, 1):
-        N.lib().ol_debug_sort_variant(variant)
-        try:
-            gk, gv = sort_pairs(keys, vals, *bits)
-        finally:
-            N.lib().ol_debug_sort_variant(0)
-        assert (gv == vals[order]).all(), f"tile shape {variant}: values out of stable order"
-        assert (gk == keys[order]).all(), f"tile shape {variant}: keys out of order"
+    gk, gv = sort_pairs(keys, vals, *bits)
+    assert (gv == vals[order]).all(), "values out of stable order"
+    assert (gk == keys[order]).all(), "keys out of order"
 
 
 @pytest.mark.parametrize("n", [4097, 250_000])

@@ -1,7 +1,7 @@
 """Helper of test_gpu_toggles.py (also runnable by hand): builds one grid on cuda:0 from seeded LiDAR scans, runs
 subdivide + RANSAC and prints a SHA-256 over every exported table.  The digest must not depend on HOW the clouds were
-handed over (pageable numpy / pinned numpy / CUDA tensors in small batches) nor on the library's internal switches
-(environment: OL_NO_EMBED, OL_RUNS_ONE_PASS, OL_NO_PREFETCH, OL_CACHE_BYTES)."""
+handed over (pageable numpy / pinned numpy / CUDA tensors in small batches) nor on the size of the library's device
+block cache (environment: OL_CACHE_BYTES)."""
 import hashlib
 import os
 import sys
