@@ -337,7 +337,8 @@ int ol_measure_fma_peak(void *stream, double *out_fp64_tflops, double *out_fp32_
  *         range} of a 1-in-8 sample of the rank's points; enqueued on the stream, not synchronised.
  * ol_partition_by_owner reorders a rank's local cloud xyz_dev ([n][3] float64, a concatenation of
  * n_segments runs = poses) into out_xyz_dev grouped by owner rank, stable inside (owner, run), and
- * returns counts[owner][run] (host, int64) - the send layout of one NCCL all-to-all. */
+ * returns counts[owner][run] (host, int64) - the send layout of one all-to-all, the exchange of the multi-GPU grid where
+ * ol_exchange_run cannot run (a backend other than NCCL, or no peer-mapped memory).  Synchronises. */
 uint32_t ol_host_cell_owner(int64_t qx, int64_t qy, int64_t qz, uint32_t world);
 int ol_slab_histogram(void *stream, const double *xyz_dev, int64_t n, double edge, double corner_x, int32_t n_bins,
                       int64_t *out_dev);
@@ -345,28 +346,6 @@ int ol_partition_by_owner(void *stream, const double *xyz_dev, int64_t n, const 
                           double edge, const double corner[3], int32_t world, const int64_t *slab_bounds_host,
                           double *out_xyz_dev, int64_t *out_counts_host, ol_alloc_fn alloc, ol_free_fn free_fn,
                           void *alloc_user);
-
-/* Fused form used when the ranks of one node can map each other's memory (NVLink peer access):
- * ol_route_plan        = the same owner computation and stable sort, but only the permutation
- *                        (out_perm_dev[i] = source row of the i-th row in (owner, run) order) and the counts are
- *                        produced - no local staging copy;
- * ol_route_to_peers    = one kernel that reads the rows in that order and stores each one directly into the receive
- *                        buffer of its owner rank (peer_base_host[o], device pointers valid in THIS process) starting
- *                        at row recv_row_base_host[o]; owner_first_host[o] = first sorted position owned by rank o
- *                        (world + 1 entries).  The caller orders it against the peers with its own barriers. */
-int ol_route_plan(void *stream, const double *xyz_dev, int64_t n, const int64_t *seg_sizes_host, int32_t n_segments, double edge,
-                  const double corner[3], int32_t world, const int64_t *slab_bounds_host, uint32_t *out_perm_dev,
-                  int64_t *out_counts_host, ol_alloc_fn alloc, ol_free_fn free_fn, void *alloc_user);
-/* ol_route_plan without any host synchronisation: the send layout stays on the device as the DENSE table
- * out_dense_dev[owner][pose number] (int64, world x n_poses_total) followed by ONE extra element, the device error word
- * (non-zero: NaN / out-of-range coordinates) - ready for one all-gather, after which every rank knows every row count.
- * seg_pose_host[s] = pose number of local run s. */
-int ol_route_plan_dev(void *stream, const double *xyz_dev, int64_t n, const int64_t *seg_sizes_host, const int32_t *seg_pose_host,
-                      int32_t n_segments, int32_t n_poses_total, double edge, const double corner[3], int32_t world,
-                      const int64_t *slab_bounds_host, uint32_t *out_perm_dev, int64_t *out_dense_dev, ol_alloc_fn alloc,
-                      ol_free_fn free_fn, void *alloc_user);
-int ol_route_to_peers(void *stream, const double *xyz_dev, const uint32_t *perm_dev, int64_t n, int32_t world,
-                      const int64_t *owner_first_host, void *const *peer_base_host, const int64_t *recv_row_base_host);
 
 /* ---- fused exchange over peer-mapped memory (csrc/exchange.cu) ----------------------------------------------------------
  * The production path of the multi-GPU grid when the ranks of a node can map each other's memory: owner rule, counting,

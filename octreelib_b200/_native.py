@@ -112,10 +112,6 @@ SIGNATURES = {
     "ol_slab_histogram": (C.c_int, [_p, _p, _i64, _f64, _f64, _i32, _p]),
     "ol_partition_by_owner": (C.c_int, [_p, _p, _i64, _p, _i32, _f64, C.POINTER(_f64 * 3), _i32, _p, _p, _p, ALLOC_FN, FREE_FN,
                                         _p]),
-    "ol_route_plan": (C.c_int, [_p, _p, _i64, _p, _i32, _f64, C.POINTER(_f64 * 3), _i32, _p, _p, _p, ALLOC_FN, FREE_FN, _p]),
-    "ol_route_plan_dev": (C.c_int, [_p, _p, _i64, _p, _p, _i32, _i32, _f64, C.POINTER(_f64 * 3), _i32, _p, _p, _p, ALLOC_FN, FREE_FN,
-                                    _p]),
-    "ol_route_to_peers": (C.c_int, [_p, _p, _p, _i64, _i32, _p, _p, _p]),
     "ol_exchange_ctrl_bytes": (_i64, [_i32, _i32]),
     "ol_exchange_create": (C.c_int, [_i32, _i32, _i32, _i64, _i32, _p, _p, _i32, C.POINTER(_p)]),
     "ol_exchange_destroy": (C.c_int, [_p]),

@@ -8,10 +8,9 @@
 //         `block_start_indices` (ransac/cuda_ransac.py:65-67) of a block is the local one plus the pose's point count on
 //         the lower ranks - exact with one small all-gather.  The boundaries are count quantiles of ix over all ranks
 //         (ol_slab_histogram + one all-gather), chosen identically by every rank.
-// The exchange is: either a staging copy for an NCCL all-to-all (ol_partition_by_owner) or
-// the fused route kernel that stores every row straight into its owner's peer-mapped receive buffer
-// over NVLink (ol_route_plan + ol_route_to_peers).  The reference has no counterpart (single process);
-// the cell coordinates are the ones of /root/reference/octreelib/grid/grid.py:72-76.
+// ol_partition_by_owner is the staged exchange, the fallback where the fused one (exchange.cu) cannot run: a staging copy
+// grouped by owner and the counts of one all-to-all.  The reference has no counterpart (single process); the cell
+// coordinates are the ones of /root/reference/octreelib/grid/grid.py:72-76.
 #include <climits>
 
 #include "common.cuh"
@@ -84,30 +83,6 @@ __global__ void route_counts_kernel(uint32_t n, const uint32_t* __restrict__ own
     const bool tail = (i == n - 1) || owner_sorted[i + 1] != o || seg_of(perm[i + 1]) != s;
     if (head) run_begin[slot] = i;
     if (tail) run_end[slot] = (unsigned long long)i + 1;
-}
-
-struct RouteArgs {
-    double* peer[ROUTE_MAX_WORLD];        // receive buffer of every rank, mapped into this process (NVLink peer memory)
-    long long base[ROUTE_MAX_WORLD];      // first row this rank may write in that buffer
-    uint32_t first[ROUTE_MAX_WORLD + 1];  // first sorted position owned by every rank
-    int world;
-};
-
-// Fused gather + all-to-all: row i of the owner-sorted order is read from the local cloud and stored straight
-// into the owning rank's receive buffer over NVLink (P2P stores; consecutive threads write consecutive rows).
-__global__ void __launch_bounds__(256) route_to_peers_kernel(const double* __restrict__ xyz, const uint32_t* __restrict__ perm,
-                                                             uint32_t n, const __grid_constant__ RouteArgs a) {
-    // one thread per DOUBLE of the routed stream: a warp instruction stores 256 contiguous bytes into the peer
-    // (row-per-thread stores of 3 x 8 B with a 24 B stride reach only ~110 GB/s over NVLink: peer stores are
-    // not merged across instructions)
-    const size_t f = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (f >= (size_t)n * 3) return;
-    const uint32_t i = (uint32_t)(f / 3);
-    const uint32_t c = (uint32_t)(f - (size_t)i * 3);
-    int o = 0;
-    while (o + 1 < a.world && a.first[o + 1] <= i) ++o;
-    const size_t r = perm[i];
-    a.peer[o][(size_t)(a.base[o] + (long long)(i - a.first[o])) * 3 + c] = xyz[r * 3 + c];
 }
 
 // ---- slab boundaries: range and histogram of the leading cell coordinate ---------------------------------------------
@@ -198,157 +173,60 @@ int ol_slab_histogram(void* stream, const double* xyz_dev, int64_t n, double edg
 
 uint32_t ol_host_cell_owner(int64_t qx, int64_t qy, int64_t qz, uint32_t world) { return ol::cell_owner(qx, qy, qz, world); }
 
-// dense send layout on the device: out[owner][pose number] += rows of every (owner, local run) pair; the error word rides
-// in the extra last element, so that ONE all-gather + ONE read-back serve every rank (no host round trip in between)
-__global__ void counts_dense_kernel(int world, int n_seg, int n_poses, const unsigned long long* __restrict__ rb,
-                                    const unsigned long long* __restrict__ re, const int32_t* __restrict__ seg_pose,
-                                    const uint32_t* __restrict__ err, long long* __restrict__ out /*[world][n_poses] + 1*/) {
-    const int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k == 0) out[(size_t)world * n_poses] = (long long)*err;
-    if (k >= world * n_seg) return;
-    const int o = k / n_seg, s = k - o * n_seg;
-    const unsigned long long cnt = re[k] - rb[k];
-    if (cnt) atomicAdd(reinterpret_cast<unsigned long long*>(&out[(size_t)o * n_poses + seg_pose[s]]), cnt);
-}
-
-// shared by ol_partition_by_owner / ol_route_plan: owner per point, stable sort by owner, (owner, run) counts.
-// out_counts_host != NULL: counts[owner][run] are read back (one synchronisation); out_dense_dev != NULL: the dense
-// [owner][pose number] layout (+ the error word) is left on the device instead, no synchronisation.
-static void route_plan(ol::Ctx& c, const double* xyz_dev, int64_t n, const int64_t* seg_sizes_host, int32_t n_segments, double edge,
-                       const double corner[3], int32_t world, const int64_t* slab_bounds_host, uint32_t* out_perm_dev,
-                       double* out_xyz_dev, int64_t* out_counts_host, const int32_t* seg_pose_host = nullptr, int32_t n_poses = 0,
-                       int64_t* out_dense_dev = nullptr) {
-    using namespace ol;
-    OL_REQUIRE(n >= 0 && n < (1ll << 31) && n_segments >= 1 && world >= 1 && world <= ROUTE_MAX_WORLD && edge > 0, OL_ERR_INVALID,
-               "bad partition arguments");
-    OwnerRule rule{};
-    if (slab_bounds_host) {
-        rule.slabs = 1;
-        for (int k = 0; k + 1 < world; ++k) {
-            OL_REQUIRE(k == 0 || slab_bounds_host[k] >= slab_bounds_host[k - 1], OL_ERR_INVALID, "slab boundaries must ascend");
-            rule.bound[k] = slab_bounds_host[k];
-        }
-    }
-    if (out_counts_host)
-        for (int64_t k = 0; k < (int64_t)world * n_segments; ++k) out_counts_host[k] = 0;
-    if (out_dense_dev) OL_CUDA(cudaMemsetAsync(out_dense_dev, 0, sizeof(int64_t) * ((size_t)world * n_poses + 1), c.stream));
-    if (n == 0) return;
-    const uint32_t m = (uint32_t)n;
-    std::vector<uint32_t> seg_start((size_t)n_segments + 1, 0);
-    for (int s = 0; s < n_segments; ++s) seg_start[s + 1] = seg_start[s] + (uint32_t)seg_sizes_host[s];
-    OL_REQUIRE(seg_start[n_segments] == m, OL_ERR_INVALID, "segment sizes do not add up to n");
-    DevBuf<uint32_t> err(c, 1), k0(c, m), k1(c, m), v0(c, m), v1(c, m), d_seg(c, seg_start.size());
-    DevBuf<unsigned long long> rb(c, (size_t)world * n_segments), re(c, (size_t)world * n_segments);
-    err.zero();
-    rb.zero();
-    re.zero();
-    h2d(c, d_seg.get(), seg_start.data(), seg_start.size());
-    const unsigned g = (m + 255) / 256;
-    owner_kernel<<<g, 256, 0, c.stream>>>(xyz_dev, m, edge, corner[0], corner[1], corner[2], (uint32_t)world, rule, k0.get(), v0.get(),
-                                          err.get());
-    OL_CHECK_LAUNCH();
-    int w = radix_sort_pairs<uint32_t>(c, k0.get(), k1.get(), v0.get(), v1.get(), m, 0, bit_length_u64((uint64_t)world - 1));
-    const uint32_t* ks = w ? k1.get() : k0.get();
-    const uint32_t* vs = w ? v1.get() : v0.get();
-    if (out_xyz_dev) {
-        route_gather_kernel<<<g, 256, 0, c.stream>>>(m, xyz_dev, vs, out_xyz_dev);
-        OL_CHECK_LAUNCH();
-    }
-    if (out_perm_dev) d2d(c, out_perm_dev, vs, m);
-    route_counts_kernel<<<g, 256, 0, c.stream>>>(m, ks, vs, d_seg.get(), n_segments, rb.get(), re.get());
-    OL_CHECK_LAUNCH();
-    if (out_dense_dev) {
-        DevBuf<int32_t> d_pose(c, (size_t)n_segments);
-        h2d(c, d_pose.get(), seg_pose_host, (size_t)n_segments);
-        counts_dense_kernel<<<(world * n_segments + 255) / 256, 256, 0, c.stream>>>(world, n_segments, n_poses, rb.get(), re.get(),
-                                                                                  d_pose.get(), err.get(), (long long*)out_dense_dev);
-        OL_CHECK_LAUNCH();
-        return;  // temporaries are released in stream order (caching allocator on the same stream)
-    }
-    std::vector<unsigned long long> hb((size_t)world * n_segments), he((size_t)world * n_segments);
-    uint32_t herr = 0;
-    d2h(c, hb.data(), rb.get(), hb.size());
-    d2h(c, he.data(), re.get(), he.size());
-    d2h(c, &herr, err.get(), 1);
-    c.sync();
-    OL_REQUIRE(!(herr & DEVERR_NONFINITE), OL_ERR_NONFINITE, "point cloud contains NaN or infinite coordinates");
-    OL_REQUIRE(!(herr & DEVERR_CELL_RANGE), OL_ERR_RANGE, "cell coordinates out of the representable range");
-    for (size_t k = 0; k < hb.size(); ++k) out_counts_host[k] = (int64_t)(he[k] - hb[k]);
-}
-
-static ol::Ctx route_ctx(void* stream, ol_alloc_fn alloc, ol_free_fn free_fn, void* alloc_user) {
-    ol::Ctx c;
-    c.stream = (cudaStream_t)stream;
-    c.alloc_fn = alloc;
-    c.free_fn = free_fn;
-    c.alloc_user = alloc_user;
-    c.pool_enabled = true;
-    return c;
-}
-
+// Owner per point, stable sort by owner, gather into that order; counts[owner][run] are read back (one synchronisation).
 int ol_partition_by_owner(void* stream, const double* xyz_dev, int64_t n, const int64_t* seg_sizes_host, int32_t n_segments,
                           double edge, const double corner[3], int32_t world, const int64_t* slab_bounds_host, double* out_xyz_dev,
                           int64_t* out_counts_host, ol_alloc_fn alloc, ol_free_fn free_fn, void* alloc_user) {
-    try {
-        ol::Ctx c = route_ctx(stream, alloc, free_fn, alloc_user);
-        route_plan(c, xyz_dev, n, seg_sizes_host, n_segments, edge, corner, world, slab_bounds_host, nullptr, out_xyz_dev,
-                   out_counts_host);
-    } catch (const ol::Error& e) {
-        ol::set_last_error(e.code, e.msg);
-        return e.code;
-    }
-    return OL_OK;
-}
-
-int ol_route_plan(void* stream, const double* xyz_dev, int64_t n, const int64_t* seg_sizes_host, int32_t n_segments, double edge,
-                  const double corner[3], int32_t world, const int64_t* slab_bounds_host, uint32_t* out_perm_dev,
-                  int64_t* out_counts_host, ol_alloc_fn alloc, ol_free_fn free_fn, void* alloc_user) {
-    try {
-        ol::Ctx c = route_ctx(stream, alloc, free_fn, alloc_user);
-        route_plan(c, xyz_dev, n, seg_sizes_host, n_segments, edge, corner, world, slab_bounds_host, out_perm_dev, nullptr,
-                   out_counts_host);
-    } catch (const ol::Error& e) {
-        ol::set_last_error(e.code, e.msg);
-        return e.code;
-    }
-    return OL_OK;
-}
-
-int ol_route_plan_dev(void* stream, const double* xyz_dev, int64_t n, const int64_t* seg_sizes_host, const int32_t* seg_pose_host,
-                      int32_t n_segments, int32_t n_poses_total, double edge, const double corner[3], int32_t world,
-                      const int64_t* slab_bounds_host, uint32_t* out_perm_dev, int64_t* out_dense_dev, ol_alloc_fn alloc,
-                      ol_free_fn free_fn, void* alloc_user) {
-    try {
-        ol::Ctx c = route_ctx(stream, alloc, free_fn, alloc_user);
-        OL_REQUIRE(seg_pose_host && out_dense_dev && n_poses_total >= 1, OL_ERR_INVALID, "bad arguments");
-        for (int s = 0; s < n_segments; ++s)
-            OL_REQUIRE(seg_pose_host[s] >= 0 && seg_pose_host[s] < n_poses_total, OL_ERR_POSE, "pose number out of range");
-        route_plan(c, xyz_dev, n, seg_sizes_host, n_segments, edge, corner, world, slab_bounds_host, out_perm_dev, nullptr, nullptr,
-                   seg_pose_host, n_poses_total, out_dense_dev);
-    } catch (const ol::Error& e) {
-        ol::set_last_error(e.code, e.msg);
-        return e.code;
-    }
-    return OL_OK;
-}
-
-int ol_route_to_peers(void* stream, const double* xyz_dev, const uint32_t* perm_dev, int64_t n, int32_t world,
-                      const int64_t* owner_first_host, void* const* peer_base_host, const int64_t* recv_row_base_host) {
     using namespace ol;
     try {
-        OL_REQUIRE(world >= 1 && world <= ROUTE_MAX_WORLD && n >= 0 && n < (1ll << 31), OL_ERR_INVALID, "bad routing arguments");
-        if (n == 0) return OL_OK;
-        RouteArgs a{};
-        a.world = world;
-        for (int o = 0; o < world; ++o) {
-            a.peer[o] = static_cast<double*>(peer_base_host[o]);
-            a.base[o] = recv_row_base_host[o];
-            a.first[o] = (uint32_t)owner_first_host[o];
+        Ctx c;
+        c.stream = (cudaStream_t)stream;
+        c.alloc_fn = alloc;
+        c.free_fn = free_fn;
+        c.alloc_user = alloc_user;
+        c.pool_enabled = true;
+        OL_REQUIRE(n >= 0 && n < (1ll << 31) && n_segments >= 1 && world >= 1 && world <= ROUTE_MAX_WORLD && edge > 0, OL_ERR_INVALID,
+                   "bad partition arguments");
+        OwnerRule rule{};
+        if (slab_bounds_host) {
+            rule.slabs = 1;
+            for (int k = 0; k + 1 < world; ++k) {
+                OL_REQUIRE(k == 0 || slab_bounds_host[k] >= slab_bounds_host[k - 1], OL_ERR_INVALID, "slab boundaries must ascend");
+                rule.bound[k] = slab_bounds_host[k];
+            }
         }
-        a.first[world] = (uint32_t)owner_first_host[world];
-        OL_REQUIRE(owner_first_host[world] == n, OL_ERR_INVALID, "owner offsets do not cover the cloud");
-        route_to_peers_kernel<<<(unsigned)(((size_t)n * 3 + 255) / 256), 256, 0, (cudaStream_t)stream>>>(xyz_dev, perm_dev, (uint32_t)n, a);
+        for (int64_t k = 0; k < (int64_t)world * n_segments; ++k) out_counts_host[k] = 0;
+        if (n == 0) return OL_OK;
+        const uint32_t m = (uint32_t)n;
+        std::vector<uint32_t> seg_start((size_t)n_segments + 1, 0);
+        for (int s = 0; s < n_segments; ++s) seg_start[s + 1] = seg_start[s] + (uint32_t)seg_sizes_host[s];
+        OL_REQUIRE(seg_start[n_segments] == m, OL_ERR_INVALID, "segment sizes do not add up to n");
+        DevBuf<uint32_t> err(c, 1), k0(c, m), k1(c, m), v0(c, m), v1(c, m), d_seg(c, seg_start.size());
+        DevBuf<unsigned long long> rb(c, (size_t)world * n_segments), re(c, (size_t)world * n_segments);
+        err.zero();
+        rb.zero();
+        re.zero();
+        h2d(c, d_seg.get(), seg_start.data(), seg_start.size());
+        const unsigned g = (m + 255) / 256;
+        owner_kernel<<<g, 256, 0, c.stream>>>(xyz_dev, m, edge, corner[0], corner[1], corner[2], (uint32_t)world, rule, k0.get(),
+                                              v0.get(), err.get());
         OL_CHECK_LAUNCH();
+        int w = radix_sort_pairs<uint32_t>(c, k0.get(), k1.get(), v0.get(), v1.get(), m, 0, bit_length_u64((uint64_t)world - 1));
+        const uint32_t* ks = w ? k1.get() : k0.get();
+        const uint32_t* vs = w ? v1.get() : v0.get();
+        route_gather_kernel<<<g, 256, 0, c.stream>>>(m, xyz_dev, vs, out_xyz_dev);
+        OL_CHECK_LAUNCH();
+        route_counts_kernel<<<g, 256, 0, c.stream>>>(m, ks, vs, d_seg.get(), n_segments, rb.get(), re.get());
+        OL_CHECK_LAUNCH();
+        std::vector<unsigned long long> hb((size_t)world * n_segments), he((size_t)world * n_segments);
+        uint32_t herr = 0;
+        d2h(c, hb.data(), rb.get(), hb.size());
+        d2h(c, he.data(), re.get(), he.size());
+        d2h(c, &herr, err.get(), 1);
+        c.sync();
+        OL_REQUIRE(!(herr & DEVERR_NONFINITE), OL_ERR_NONFINITE, "point cloud contains NaN or infinite coordinates");
+        OL_REQUIRE(!(herr & DEVERR_CELL_RANGE), OL_ERR_RANGE, "cell coordinates out of the representable range");
+        for (size_t k = 0; k < hb.size(); ++k) out_counts_host[k] = (int64_t)(he[k] - hb[k]);
     } catch (const ol::Error& e) {
         ol::set_last_error(e.code, e.msg);
         return e.code;

@@ -6,7 +6,7 @@ is per (pose, leaf) block, cuda_ransac.py:94-97), so the grid shards by CELL, by
 
     partition="slab" (default)  owner(cell) = #{k : bound[k] <= ix}: an ORDER-PRESERVING hash of the cell key.  The
                                 world - 1 boundaries are count quantiles of the leading cell coordinate over all ranks
-                                (`ol_slab_histogram` + one all-gather), so the load is balanced, and because the reference
+                                (a sample histogram per rank), so the load is balanced, and because the reference
                                 enumerates cells lexicographically (grid/grid.py:79-81) every cell of rank r precedes every
                                 cell of rank r + 1.  That makes the two things that depend on the GLOBAL order exact: the
                                 batch layout of the RANSAC kernel (`block_start_indices`, cuda_ransac.py:65-67: the sample
@@ -17,11 +17,13 @@ is per (pose, leaf) block, cuda_ransac.py:94-97), so the grid shards by CELL, by
                                 it the sample index where `R n + start` sits within an ulp of an integer (p ~ 1e-8 per
                                 draw) - would need a merge of all (cell, pose) tables.
 
-`ShardedGrid.insert_points` stages a rank's local clouds; `exchange()` partitions them by owner on the
-GPU (`ol_partition_by_owner`: owner kernel + stable radix sort + gather), moves them with ONE
-all-to-all (counts first) and inserts what arrived as (source rank, pose) runs.  After that every
-operation is local to the rank - there is no further data-path collective; only scalar counters and
-the final leaf / plane tables are reduced or gathered.
+`ShardedGrid.insert_points` stages a rank's local clouds; `exchange()` moves every point to the rank that owns its cell.
+On one rank, or in an NCCL group whose ranks map each other's memory (torch symmetric memory), that is the fused exchange
+of csrc/exchange.cu (`_FusedExchange`): owner rule, counting and peer stores over NVLink in one native call, after which
+the receiving forest adopts the receive buffer.  Elsewhere - another backend, or no symmetric memory - the staged exchange
+runs: `ol_partition_by_owner` (owner kernel + stable radix sort + gather), ONE all-to-all (counts first), and insertion of
+what arrived as (source rank, pose) runs.  After that every operation is local to the rank - there is no further
+data-path collective; only scalar counters and the final leaf / plane tables are reduced or gathered.
 
 The routing helpers (`routing_layout`, `exchange_points`) are device independent so that the host
 logic is covered by world_size-2 `gloo` tests on CPU.
@@ -126,45 +128,6 @@ def segments_from_counts(recv_counts: np.ndarray) -> Tuple[np.ndarray, np.ndarra
     before = np.cumsum(rc, axis=0) - rc
     src, pose = np.nonzero(rc)  # row-major: source rank, then pose -> the order of the received buffer
     return rc[src, pose].astype(np.int64), pose.astype(np.int32), before[src, pose].astype(np.int64)
-
-
-class _PeerBuffers:
-    """Symmetric receive buffers (torch.distributed._symmetric_memory: every rank's buffer is mapped into every
-    process of the node, so a kernel can store into a peer over NVLink).  One set per (group, capacity), reused
-    by every ShardedGrid of the process."""
-
-    _cache: Dict[Tuple[int, int], "_PeerBuffers"] = {}
-    disabled_reason: Optional[str] = None
-
-    def __init__(self, rows: int, device, group):
-        import torch
-        import torch.distributed as dist
-        import torch.distributed._symmetric_memory as symm
-
-        self.rows = rows
-        self.buf = symm.empty(rows * 3, dtype=torch.float64, device=device)
-        self.hdl = symm.rendezvous(self.buf, group if group is not None else dist.group.WORLD)
-        self.ptrs = [int(p) for p in self.hdl.buffer_ptrs]
-
-    @classmethod
-    def get(cls, rows_needed: int, device, group, world: int) -> Optional["_PeerBuffers"]:
-        """Collective: every rank calls it with the same rows_needed."""
-        if cls.disabled_reason is not None:
-            return None
-        best = None
-        for (w, rows), pb in cls._cache.items():
-            if w == world and rows >= rows_needed and (best is None or rows < best.rows):
-                best = pb
-        if best is not None:
-            return best
-        try:
-            rows = int(rows_needed * 1.25) + 4096
-            pb = cls(rows, device, group)
-        except Exception as exc:  # noqa: BLE001 - symmetric memory unavailable: stay on the NCCL all-to-all
-            cls.disabled_reason = f"{type(exc).__name__}: {exc}"
-            return None
-        cls._cache[(world, rows)] = pb
-        return pb
 
 
 class _FusedExchange:
@@ -310,160 +273,24 @@ class ShardedGrid:
         self._staged.append((int(pose_number), points))
 
     def exchange(self):
-        """Route every staged point to the rank that owns its cell (one NCCL all-to-all)."""
-        import os
-        import time
-        torch = require_cuda()
-        timing = os.environ.get("OL_TIMING") == "1"
-        marks = []
-
-        host_only = os.environ.get("OL_TIMING") == "host"  # host wall time per phase, no device synchronisation
-        timing = timing or host_only
-
-        def mark(name):
-            if timing:
-                if not host_only:
-                    torch.cuda.synchronize()
-                marks.append((name, time.perf_counter()))
-
-        mark("start")
-        lib = N.lib()
+        """Route every staged point to the rank that owns its cell.  The fused exchange runs wherever it can: on a single
+        rank, or in an NCCL group whose ranks map each other's memory.  Otherwise (another backend, or
+        `_FusedExchange.disabled_reason` set because symmetric memory is unavailable) the staged all-to-all runs."""
+        if any(a[0] > b[0] for a, b in zip(self._staged, self._staged[1:])):
+            self._staged.sort(key=lambda s: s[0])  # stable: poses ascending, insertion order inside a pose
         dev = self._host.forest.device
-        stream = torch.cuda.current_stream(dev)
-        mode = os.environ.get("OL_EXCHANGE", "fused")
-        if (mode == "fused" and _FusedExchange.disabled_reason is None and not self.exchanged
+        if (_FusedExchange.disabled_reason is None and not self.exchanged
                 and (self.world == 1 or self._dist.get_backend(self._group) == "nccl")):
-            if self._exchange_fused(dev, mark):
-                if timing and self.rank == 0:
-                    print("[exchange fused] " + ", ".join(f"{b[0]} {1e3 * (b[1] - a[1]):.2f} ms" for a, b in zip(marks, marks[1:])),
-                          flush=True)
+            if self._exchange_fused(dev):
                 return
-        parts = []
-        for _, pts in self._staged:
-            t = pts if isinstance(pts, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(pts, dtype=np.float64))
-            parts.append(t.to(dev, dtype=torch.float64, non_blocking=True).reshape(-1, 3))
-        numbers = [p for p, _ in self._staged]
-        sizes = np.array([int(t.shape[0]) for t in parts] or [0], dtype=np.int64)
-        local = torch.cat(parts) if parts else torch.empty((0, 3), dtype=torch.float64, device=dev)
-        mark("stage")
-        n, n_seg = int(local.shape[0]), max(len(parts), 1)
-        counts = np.zeros((self.world, n_seg), dtype=np.int64)
-        alloc = TorchAllocator(dev)
-        corner = (C.c_double * 3)(*self._corner)
-        bounds = None
-        if self.partition == "slab" and self.world > 1:
-            # count quantiles of the leading cell coordinate over all ranks: one small all-gather, one read-back
-            hist = torch.empty(2 + SLAB_BINS, dtype=torch.int64, device=dev)
-            N.check(lib.ol_slab_histogram(C.c_void_p(stream.cuda_stream), C.c_void_p(local.data_ptr()), n,
-                                          float(self._cfg.voxel_edge_length), float(self._corner[0]), SLAB_BINS,
-                                          C.c_void_p(hist.data_ptr())))
-            allh = torch.empty((self.world, 2 + SLAB_BINS), dtype=torch.int64, device=dev)
-            self._dist.all_gather_into_tensor(allh, hist, group=self._group)
-            self.slab_bounds = slab_boundaries(allh.cpu().numpy(), self.world)
-            bounds = np.ascontiguousarray(self.slab_bounds, dtype=np.int64)
-            mark("slabs")
-        bounds_p = None if bounds is None else bounds.ctypes.data_as(C.c_void_p)
-        use_p2p = self.world > 1 and mode in ("fused", "p2p") and self._dist.get_backend(self._group) == "nccl"
-        perm = send = None
-        recv = None
-        send_counts = None
+        self._exchange_staged(dev)
 
-        def staged_partition():
-            """owner-grouped staging copy + counts on the host (the NCCL all-to-all path)"""
-            nonlocal send, send_counts
-            send = torch.empty_like(local)
-            N.check(lib.ol_partition_by_owner(C.c_void_p(stream.cuda_stream), C.c_void_p(local.data_ptr()), n,
-                                              sizes.ctypes.data_as(C.c_void_p), n_seg, float(self._cfg.voxel_edge_length),
-                                              C.byref(corner), self.world, bounds_p, C.c_void_p(send.data_ptr()),
-                                              counts.ctypes.data_as(C.c_void_p), alloc.alloc_cb, alloc.free_cb, None))
-            send_counts = routing_layout(counts[:, :len(parts)] if parts else counts[:, :0], numbers, self.n_poses_total)
-
-        if use_p2p:
-            # Owner sort and (owner, pose) row counts stay on the device; the dense send layout of every rank (+ its error
-            # word) is all-gathered and read back ONCE: every rank then knows the whole (source, destination, pose) cube.
-            perm = torch.empty(max(n, 1), dtype=torch.int32, device=dev)
-            mine = torch.empty(self.world * self.n_poses_total + 1, dtype=torch.int64, device=dev)
-            seg_pose_local = np.ascontiguousarray(numbers if numbers else [0], dtype=np.int32)
-            N.check(lib.ol_route_plan_dev(C.c_void_p(stream.cuda_stream), C.c_void_p(local.data_ptr()), n,
-                                          sizes.ctypes.data_as(C.c_void_p), seg_pose_local.ctypes.data_as(C.c_void_p), n_seg,
-                                          self.n_poses_total, float(self._cfg.voxel_edge_length), C.byref(corner), self.world, bounds_p,
-                                          C.c_void_p(perm.data_ptr()), C.c_void_p(mine.data_ptr()), alloc.alloc_cb, alloc.free_cb, None))
-            mark("partition")
-            cube_t = torch.empty((self.world, mine.shape[0]), dtype=torch.int64, device=dev)
-            self._dist.all_gather_into_tensor(cube_t, mine, group=self._group)
-            gathered = cube_t.cpu().numpy()
-            if gathered[:, -1].any():
-                bad = int(np.bitwise_or.reduce(gathered[:, -1]))
-                raise ValueError("point cloud contains NaN or infinite coordinates" if bad & 1 else
-                                 "cell coordinates out of the representable range")
-            cube = gathered[:, :-1].reshape(self.world, self.world, self.n_poses_total)   # [src][dst][pose]
-            send_counts = cube[self.rank]
-            tot = cube.sum(axis=2)                           # [src][dst]
-            pb = _PeerBuffers.get(int(tot.sum(axis=0).max()), dev, self._group, self.world)
-            if pb is None:
-                use_p2p = False
-                staged_partition()
-            else:
-                owner_first = np.concatenate([[0], np.cumsum(send_counts.sum(axis=1))]).astype(np.int64)
-                base = (np.cumsum(tot, axis=0) - tot)[self.rank].astype(np.int64)   # rows of lower source ranks, per destination
-                ptrs = (C.c_void_p * self.world)(*pb.ptrs)
-                ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)] if (timing and not host_only) else None
-                mark("allgather")
-                if ev:
-                    ev[0].record()
-                pb.hdl.barrier()                             # the peers have consumed what the previous exchange delivered
-                if ev:
-                    ev[1].record()
-                mark("barrier0")
-                N.check(lib.ol_route_to_peers(C.c_void_p(stream.cuda_stream), C.c_void_p(local.data_ptr()),
-                                              C.c_void_p(perm.data_ptr()), n, self.world, owner_first.ctypes.data_as(C.c_void_p),
-                                              ptrs, base.ctypes.data_as(C.c_void_p)))
-                if ev:
-                    ev[2].record()
-                mark("route")
-                pb.hdl.barrier()                             # every rank's rows have landed
-                mark("barrier1")
-                if ev:
-                    ev[3].record()
-                    torch.cuda.synchronize()
-                    if self.rank == 0:
-                        print(f"[p2p] barrier0 {ev[0].elapsed_time(ev[1]):.3f} ms, route kernel {ev[1].elapsed_time(ev[2]):.3f} ms, "
-                              f"barrier1 {ev[2].elapsed_time(ev[3]):.3f} ms", flush=True)
-                recv_counts = cube[:, self.rank, :]
-                recv = pb.buf[: int(recv_counts.sum()) * 3].view(-1, 3)
-        else:
-            staged_partition()
-            mark("partition")
-        if not use_p2p:
-            if self.world > 1:
-                recv, recv_counts = exchange_points(send, send_counts, self._group)
-            else:
-                recv, recv_counts = send, send_counts
-        mark("all_to_all")
-        seg_sizes, seg_pose, seg_first = segments_from_counts(recv_counts)
-        mark("segments")
-        if len(seg_sizes) == 0:
-            seg_sizes, seg_pose, seg_first = np.array([0], np.int64), np.array([0], np.int32), np.array([0], np.int64)
-        self._host.forest.insert_segments(recv, seg_sizes, seg_pose, seg_first, self.n_poses_total)
-        self.last_exchange = dict(sent=int(send_counts.sum() - send_counts[self.rank].sum()), received=int(recv.shape[0]),
-                                  kept=int(send_counts[self.rank].sum()), mode="p2p" if use_p2p else ("nccl" if self.world > 1 else "local"),
-                                  partition=self.partition, disabled_reason=_PeerBuffers.disabled_reason,
-                                  bytes=int(send_counts.sum() - send_counts[self.rank].sum()) * 24)
-        self._staged = []
-        self.exchanged = True
-        mark("insert")
-        if timing and self.rank == 0:
-            print("[exchange] " + ", ".join(f"{b[0]} {1e3 * (b[1] - a[1]):.2f} ms" for a, b in zip(marks, marks[1:])), flush=True)
-
-    def _exchange_fused(self, dev, mark) -> bool:
+    def _exchange_fused(self, dev) -> bool:
         """The production path (csrc/exchange.cu): one native call, no library collective, one host wait.  Returns False
-        when peer-mapped memory is not available (the caller falls back to the staged paths below)."""
+        when peer-mapped memory is not available (the caller falls back to `_exchange_staged`)."""
         torch = require_cuda()
         staged = self._staged
         numbers = [s[0] for s in staged]
-        if any(a > b for a, b in zip(numbers, numbers[1:])):
-            staged = sorted(staged, key=lambda s: s[0])  # stable: poses ascending, insertion order inside a pose
-            numbers = [s[0] for s in staged]
         # the host time of this loop is time the GPU idles: one attribute test per cloud on the fast path
         tensors, f64, dev_index = [], torch.float64, dev.index
         for _, pts in staged:
@@ -474,7 +301,6 @@ class ShardedGrid:
                 t = t.to(dev, dtype=torch.float64, non_blocking=True).contiguous().reshape(-1, 3)
             tensors.append(t)
         n_local = sum([t.shape[0] for t in tensors])
-        mark("stage")
         forest = self._host.forest
         slabs = self.partition == "slab"
         min_rows = 0
@@ -491,7 +317,6 @@ class ShardedGrid:
                 min_rows = int(xc.last_info[3])  # the same on every rank: everybody grows alike
         else:
             raise RuntimeError("exchange buffers could not be sized")
-        mark("exchange")
         if slabs and self.world > 1:
             self.slab_bounds = bounds.copy()
         self._pose_sizes = psz.astype(np.int64)
@@ -500,6 +325,56 @@ class ShardedGrid:
         self._staged = []
         self.exchanged = True
         return True
+
+    def _exchange_staged(self, dev):
+        """The fallback: an owner-grouped staging copy with counts on the host (`ol_partition_by_owner`), one all-to-all
+        of any backend (`exchange_points`), and insertion of what arrived as (source rank, pose) runs."""
+        torch = require_cuda()
+        lib = N.lib()
+        stream = torch.cuda.current_stream(dev)
+        parts = []
+        for _, pts in self._staged:
+            t = pts if isinstance(pts, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(pts, dtype=np.float64))
+            parts.append(t.to(dev, dtype=torch.float64, non_blocking=True).reshape(-1, 3))
+        numbers = [p for p, _ in self._staged]
+        sizes = np.array([int(t.shape[0]) for t in parts] or [0], dtype=np.int64)
+        local = torch.cat(parts) if parts else torch.empty((0, 3), dtype=torch.float64, device=dev)
+        n, n_seg = int(local.shape[0]), max(len(parts), 1)
+        bounds = None
+        if self.partition == "slab" and self.world > 1:
+            # count quantiles of the leading cell coordinate over all ranks: one small all-gather, one read-back
+            hist = torch.empty(2 + SLAB_BINS, dtype=torch.int64, device=dev)
+            N.check(lib.ol_slab_histogram(C.c_void_p(stream.cuda_stream), C.c_void_p(local.data_ptr()), n,
+                                          float(self._cfg.voxel_edge_length), float(self._corner[0]), SLAB_BINS,
+                                          C.c_void_p(hist.data_ptr())))
+            allh = torch.empty((self.world, 2 + SLAB_BINS), dtype=torch.int64, device=dev)
+            self._dist.all_gather_into_tensor(allh, hist, group=self._group)
+            self.slab_bounds = slab_boundaries(allh.cpu().numpy(), self.world)
+            bounds = np.ascontiguousarray(self.slab_bounds, dtype=np.int64)
+        bounds_p = None if bounds is None else bounds.ctypes.data_as(C.c_void_p)
+        send = torch.empty_like(local)
+        counts = np.zeros((self.world, n_seg), dtype=np.int64)
+        alloc = TorchAllocator(dev)
+        corner = (C.c_double * 3)(*self._corner)
+        N.check(lib.ol_partition_by_owner(C.c_void_p(stream.cuda_stream), C.c_void_p(local.data_ptr()), n,
+                                          sizes.ctypes.data_as(C.c_void_p), n_seg, float(self._cfg.voxel_edge_length),
+                                          C.byref(corner), self.world, bounds_p, C.c_void_p(send.data_ptr()),
+                                          counts.ctypes.data_as(C.c_void_p), alloc.alloc_cb, alloc.free_cb, None))
+        send_counts = routing_layout(counts[:, :len(parts)], numbers, self.n_poses_total)
+        if self.world > 1:
+            recv, recv_counts = exchange_points(send, send_counts, self._group)
+        else:
+            recv, recv_counts = send, send_counts
+        seg_sizes, seg_pose, seg_first = segments_from_counts(recv_counts)
+        if len(seg_sizes) == 0:
+            seg_sizes, seg_pose, seg_first = np.array([0], np.int64), np.array([0], np.int32), np.array([0], np.int64)
+        self._host.forest.insert_segments(recv, seg_sizes, seg_pose, seg_first, self.n_poses_total)
+        sent, kept = int(send_counts.sum() - send_counts[self.rank].sum()), int(send_counts[self.rank].sum())
+        self.last_exchange = dict(sent=sent, received=int(recv.shape[0]), kept=kept, mode="nccl" if self.world > 1 else "local",
+                                  partition=self.partition, disabled_reason=_FusedExchange.disabled_reason,
+                                  bytes=sent * 24)
+        self._staged = []
+        self.exchanged = True
 
     # ---- local pipeline -------------------------------------------------------------------------
     def subdivide(self, subdivision_criteria, pose_numbers: Optional[Sequence[int]] = None):

@@ -224,105 +224,77 @@ def test_append_to_existing_pose_in_a_manager():
         assert mp.n_nodes(p) == og.n_nodes(p) and mp.n_points(p) == og.n_points(p)
 
 
-def test_fused_route_to_peers_matches_partition():
-    """ol_route_plan + ol_route_to_peers (the fused gather + all-to-all kernel): with the 'peer' receive buffers
-    emulated by separate buffers on one device, what lands in them equals the owner-grouped staging copy of
-    ol_partition_by_owner, at the row offsets the count cube prescribes."""
-    import torch
-
-    lib = N.lib()
-    dev = torch.device("cuda", 0)
-    rng = np.random.default_rng(5)
-    clouds = [(rng.random((2500 + 300 * k, 3)) * 30 - 15).astype(np.float32).astype(np.float64) for k in range(4)]
-    world = 4
-    want_send, counts = _partition(clouds, 1.0, world)
-    local = torch.from_numpy(np.vstack(clouds)).to(dev)
-    n = len(local)
-    sizes = np.array([len(c) for c in clouds], dtype=np.int64)
-    perm = torch.empty(n, dtype=torch.int32, device=dev)
-    counts2 = np.zeros_like(counts)
-    alloc = TorchAllocator(dev)
-    corner = (C.c_double * 3)(0.0, 0.0, 0.0)
-    stream = torch.cuda.current_stream(dev)
-    N.check(lib.ol_route_plan(C.c_void_p(stream.cuda_stream), C.c_void_p(local.data_ptr()), n, sizes.ctypes.data_as(C.c_void_p),
-                              len(sizes), 1.0, C.byref(corner), world, None, C.c_void_p(perm.data_ptr()),
-                              counts2.ctypes.data_as(C.c_void_p), alloc.alloc_cb, alloc.free_cb, None))
-    assert (counts2 == counts).all()
-    per_owner = counts.sum(axis=1)
-    owner_first = np.concatenate([[0], np.cumsum(per_owner)]).astype(np.int64)
-    base = np.array([7, 0, 3, 11], dtype=np.int64)  # as if lower source ranks had already claimed these rows
-    bufs = [torch.full((int(per_owner[o] + base[o]) * 3 + 3,), -1.0, dtype=torch.float64, device=dev) for o in range(world)]
-    ptrs = (C.c_void_p * world)(*[b.data_ptr() for b in bufs])
-    N.check(lib.ol_route_to_peers(C.c_void_p(stream.cuda_stream), C.c_void_p(local.data_ptr()), C.c_void_p(perm.data_ptr()), n, world,
-                                  owner_first.ctypes.data_as(C.c_void_p), ptrs, base.ctypes.data_as(C.c_void_p)))
-    torch.cuda.synchronize()
-    for o in range(world):
-        got = bufs[o].cpu().numpy()
-        lo, hi = int(base[o]) * 3, int(base[o] + per_owner[o]) * 3
-        assert (got[:lo] == -1.0).all() and (got[hi:] == -1.0).all(), "wrote outside the assigned rows"
-        assert (got[lo:hi].reshape(-1, 3) == want_send[owner_first[o]:owner_first[o + 1]]).all()
-
-
 def test_fused_exchange_world1_equals_plain_grid(monkeypatch):
     """The fused exchange (csrc/exchange.cu: count pass, scatter pass, adopted receive buffer, cell range without a bounding
-    box pass) with a single rank must reproduce a plain Grid: same blocks, same points in the same order, same planes.
-    Clouds are staged out of pose order and one pose arrives in two pieces."""
+    box pass) with a single rank must reproduce a plain Grid: same blocks, same points in the same order, same planes, same
+    counters - and so must the staged exchange it falls back to when `_FusedExchange.disabled_reason` is set.  Clouds are
+    staged out of pose order and one pose arrives in two pieces."""
     import torch
 
-    from octreelib_b200.parallel import ShardedGrid
+    from octreelib_b200.parallel import ShardedGrid, _FusedExchange
 
-    monkeypatch.setenv("OL_EXCHANGE", "fused")
     P = 5
     clouds = {p: lidar64_scan(p, seed=3)[::4] for p in range(P)}
     dev = torch.device("cuda", 0)
-    for partition in ("slab", "hash"):
-        for repeat in range(3):  # the receive buffers alternate; the third grid reuses the first one's
-            g = ShardedGrid(GridConfig(voxel_edge_length=1.0), P, partition=partition)
-            for p in (3, 0, 4, 1):
-                g.insert_points(p, torch.from_numpy(clouds[p]).to(dev) if p % 2 else clouds[p])
-            half = len(clouds[2]) // 2
-            g.insert_points(2, clouds[2][:half])
-            g.insert_points(2, clouds[2][half:])
-            g.exchange()
-            assert g.last_exchange["mode"] == "local" and g.last_exchange["received"] == sum(len(c) for c in clouds.values())
-            g.subdivide([MaxPoints(50)])
-            ref = Grid(GridConfig(voxel_edge_length=1.0))
-            for p in range(P):
-                ref.insert_points(p, clouds[p])
-            ref.subdivide([MaxPoints(50)])
-            for f_a, f_b in ((g._host.forest, ref._host.forest),):
-                la, lb = f_a.export_leaves(), f_b.export_leaves()
-                assert (la["corner"] == lb["corner"]).all() and (la["edge"] == lb["edge"]).all()
-                ba, bb = f_a.export_blocks(list(range(P))), f_b.export_blocks(list(range(P)))
-                for k in ("pose", "leaf", "size"):
-                    assert (ba[k] == bb[k]).all()
-                pa = f_a.export_points(-1, order=0, pose_rank=list(range(P)))
-                pb = f_b.export_points(-1, order=0, pose_rank=list(range(P)))
-                assert (pa["xyz"] == pb["xyz"]).all() and (pa["idx"] == pb["idx"]).all()
-            np.random.seed(11)
-            g.map_leaf_points_cuda_ransac(poses_per_batch=2, threshold=0.02, hypotheses_number=128)
-            np.random.seed(11)
-            ref.map_leaf_points_cuda_ransac(poses_per_batch=2, threshold=0.02, hypotheses_number=128)
-            ra, rb = g._host.forest.export_ransac(scored_only=True), ref._host.forest.export_ransac(scored_only=True)
-            for k in ("pose", "leaf", "size", "best", "best_count"):
-                assert (ra[k] == rb[k]).all()
-            assert (ra["plane"].view(np.uint32) == rb["plane"].view(np.uint32)).all()
-            assert [g.n_points(p) for p in range(P)] == [ref.n_points(p) for p in range(P)]
-            if repeat == 0:
-                keep = g  # stays alive across the next two exchanges: must be told to copy its points out
-    assert [keep.n_points(p) for p in range(P)] == [ref.n_points(p) for p in range(P)]
-    pk = keep._host.forest.export_points(-1, order=0, pose_rank=list(range(P)))
-    pr = ref._host.forest.export_points(-1, order=0, pose_rank=list(range(P)))
-    assert (pk["xyz"] == pr["xyz"]).all()
+    for reason in (None, "RuntimeError: no symmetric memory"):  # the fused exchange, then the staged fallback
+        with monkeypatch.context() as m:
+            if reason is not None:
+                m.setattr(_FusedExchange, "disabled_reason", reason)
+            for partition in ("slab", "hash"):
+                # the fused receive buffers alternate: the third grid reuses the first one's
+                for repeat in range(3 if reason is None else 1):
+                    g = ShardedGrid(GridConfig(voxel_edge_length=1.0), P, partition=partition)
+                    for p in (3, 0, 4, 1):
+                        g.insert_points(p, torch.from_numpy(clouds[p]).to(dev) if p % 2 else clouds[p])
+                    half = len(clouds[2]) // 2
+                    g.insert_points(2, clouds[2][:half])
+                    g.insert_points(2, clouds[2][half:])
+                    g.exchange()
+                    assert g.last_exchange["mode"] == "local" and g.last_exchange["received"] == sum(len(c) for c in clouds.values())
+                    assert g.last_exchange["disabled_reason"] == reason
+                    g.subdivide([MaxPoints(50)])
+                    ref = Grid(GridConfig(voxel_edge_length=1.0))
+                    for p in range(P):
+                        ref.insert_points(p, clouds[p])
+                    ref.subdivide([MaxPoints(50)])
+                    f_a, f_b = g._host.forest, ref._host.forest
+                    la, lb = f_a.export_leaves(), f_b.export_leaves()
+                    assert (la["corner"] == lb["corner"]).all() and (la["edge"] == lb["edge"]).all()
+                    ba, bb = f_a.export_blocks(list(range(P))), f_b.export_blocks(list(range(P)))
+                    for k in ("pose", "leaf", "size"):
+                        assert (ba[k] == bb[k]).all()
+                    pa = f_a.export_points(-1, order=0, pose_rank=list(range(P)))
+                    pb = f_b.export_points(-1, order=0, pose_rank=list(range(P)))
+                    assert (pa["xyz"] == pb["xyz"]).all() and (pa["idx"] == pb["idx"]).all()
+                    np.random.seed(11)
+                    g.map_leaf_points_cuda_ransac(poses_per_batch=2, threshold=0.02, hypotheses_number=128)
+                    np.random.seed(11)
+                    ref.map_leaf_points_cuda_ransac(poses_per_batch=2, threshold=0.02, hypotheses_number=128)
+                    ra, rb = g._host.forest.export_ransac(scored_only=True), ref._host.forest.export_ransac(scored_only=True)
+                    for k in ("pose", "leaf", "size", "best", "best_count"):
+                        assert (ra[k] == rb[k]).all()
+                    assert (ra["plane"].view(np.uint32) == rb["plane"].view(np.uint32)).all()
+                    assert [g.n_points(p) for p in range(P)] == [ref.n_points(p) for p in range(P)]
+                    if repeat == 0:
+                        keep = g  # stays alive across the next two exchanges: must be told to copy its points out
+            if reason is None:
+                assert [keep.n_points(p) for p in range(P)] == [ref.n_points(p) for p in range(P)]
+                pk = keep._host.forest.export_points(-1, order=0, pose_rank=list(range(P)))
+                pr = ref._host.forest.export_points(-1, order=0, pose_rank=list(range(P)))
+                assert (pk["xyz"] == pr["xyz"]).all()
 
 
 def test_fused_exchange_rejects_nonfinite(monkeypatch):
-    from octreelib_b200.parallel import ShardedGrid
+    """Non-finite coordinates are rejected by the fused exchange and by the staged fallback alike."""
+    from octreelib_b200.parallel import ShardedGrid, _FusedExchange
 
-    monkeypatch.setenv("OL_EXCHANGE", "fused")
-    g = ShardedGrid(GridConfig(voxel_edge_length=1.0), 1)
-    pts = np.random.default_rng(0).normal(0, 3, (1000, 3))
-    pts[17, 1] = np.nan
-    g.insert_points(0, pts)
-    with pytest.raises(ValueError, match="NaN or infinite"):
-        g.exchange()
+    for reason in (None, "RuntimeError: no symmetric memory"):  # the fused exchange, then the staged fallback
+        with monkeypatch.context() as m:
+            if reason is not None:
+                m.setattr(_FusedExchange, "disabled_reason", reason)
+            g = ShardedGrid(GridConfig(voxel_edge_length=1.0), 1)
+            pts = np.random.default_rng(0).normal(0, 3, (1000, 3))
+            pts[17, 1] = np.nan
+            g.insert_points(0, pts)
+            with pytest.raises(ValueError, match="NaN or infinite"):
+                g.exchange()

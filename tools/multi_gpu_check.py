@@ -3,12 +3,13 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 tools/multi_gpu_check.py
 
 Every rank holds a slice of the poses of a synthetic multi-pose LiDAR map.  The sharded pipeline (routing by cell owner
--> local subdivide -> local RANSAC) runs with the slab partition (fused peer-to-peer exchange kernel, and the NCCL
-all-to-all) and with the hash partition, and rank 0 compares the union of the per-rank leaf / plane tables with a plain
-single-GPU Grid built from ALL poses: same leaves (corner, edge), same (pose, leaf) blocks with the same points in the
-same order, same fitted planes (bit patterns), same per-pose counters.  poses_per_batch = 10 (the reference's default,
-3 batches here): the slab runs reproduce the reference's batch-global block starts across the ranks, and their gathered
-tables (`gather_tables`) equal the single-GPU tables row for row.
+-> local subdivide -> local RANSAC) runs on both exchange paths - the fused peer-to-peer exchange, and the staged NCCL
+all-to-all it falls back to when `_FusedExchange.disabled_reason` is set - each with the slab and the hash partition, and
+rank 0 compares the union of the per-rank leaf / plane tables with a plain single-GPU Grid built from ALL poses: same
+leaves (corner, edge), same (pose, leaf) blocks with the same points in the same order, same fitted planes (bit
+patterns), same per-pose counters.  poses_per_batch = 10 (the reference's default, 3 batches here): the slab runs
+reproduce the reference's batch-global block starts across the ranks, and their gathered tables (`gather_tables`)
+equal the single-GPU tables row for row.
 """
 import os
 import sys
@@ -20,7 +21,7 @@ import torch.distributed as dist
 
 from octreelib_b200.criteria import MaxPoints
 from octreelib_b200.grid import Grid, GridConfig
-from octreelib_b200.parallel import ShardedGrid, _FusedExchange, _PeerBuffers
+from octreelib_b200.parallel import ShardedGrid, _FusedExchange
 from octreelib_b200.synthetic import lidar64_scan
 
 rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
@@ -50,12 +51,17 @@ def plane_table(forest):
             for i, (p, l) in enumerate(zip(r["pose"], r["leaf"]))}
 
 
-def sharded(mode, partition):
-    os.environ["OL_EXCHANGE"] = mode
+def sharded(path, partition):
     g = ShardedGrid(GridConfig(voxel_edge_length=1.0), P, partition=partition)
     for p in mine:
         g.insert_points(p, clouds[p])
-    g.exchange()
+    saved = _FusedExchange.disabled_reason
+    if path == "fallback":  # the same on every rank: all of them take the staged exchange
+        _FusedExchange.disabled_reason = "fallback run of multi_gpu_check"
+    try:
+        g.exchange()
+    finally:
+        _FusedExchange.disabled_reason = saved
     g.subdivide([MaxPoints(60)])
     before = block_table(g._host.forest, P)
     np.random.seed(5)
@@ -70,8 +76,8 @@ def sharded(mode, partition):
     return gathered, counts, tables
 
 
-results = {(mode, part): sharded(mode, part) for mode, part in (("fused", "slab"), ("fused", "hash"), ("p2p", "slab"), ("nccl", "slab"),
-                                                                  ("p2p", "hash"))}
+results = {(path, part): sharded(path, part) for path, part in (("fused", "slab"), ("fused", "hash"), ("fallback", "slab"),
+                                                                  ("fallback", "hash"))}
 if rank == 0:
     def single(ppb):
         ref = Grid(GridConfig(voxel_edge_length=1.0))
@@ -87,7 +93,7 @@ if rank == 0:
                     table=ref._host.forest.export_ransac(scored_only=True))
 
     refs = {PPB: single(PPB), P: single(P)}
-    for (mode, part), (gathered, counts, tables) in results.items():
+    for (path, part), (gathered, counts, tables) in results.items():
         ref = refs[PPB if part == "slab" else P]
         union_before, union_after, union_planes = {}, {}, {}
         for g in gathered:
@@ -95,20 +101,21 @@ if rank == 0:
             union_before.update(g["before"])
             union_after.update(g["after"])
             union_planes.update(g["planes"])
-        assert union_before == ref["before"], f"{mode}/{part}: blocks after subdivide differ from the single-GPU grid"
-        assert set(union_planes) == set(ref["planes"]), f"{mode}/{part}: fitted block sets differ"
-        assert union_planes == ref["planes"], f"{mode}/{part}: planes differ"
-        assert union_after == ref["after"], f"{mode}/{part}: inlier sets differ"
-        assert counts == ref["counts"], f"{mode}/{part}: counters differ"
+        assert union_before == ref["before"], f"{path}/{part}: blocks after subdivide differ from the single-GPU grid"
+        assert set(union_planes) == set(ref["planes"]), f"{path}/{part}: fitted block sets differ"
+        assert union_planes == ref["planes"], f"{path}/{part}: planes differ"
+        assert union_after == ref["after"], f"{path}/{part}: inlier sets differ"
+        assert counts == ref["counts"], f"{path}/{part}: counters differ"
         if part == "slab":  # the gathered tables are the single-GPU tables, row for row
             assert (tables["leaves"]["corner"] == ref["leaves"]["corner"]).all() and (tables["leaves"]["edge"] == ref["leaves"]["edge"]).all()
             for k in ("pose", "leaf", "size", "best", "best_count"):
-                assert (tables["planes"][k] == ref["table"][k]).all(), f"{mode}/{part}: gathered plane table column {k} differs"
+                assert (tables["planes"][k] == ref["table"][k]).all(), f"{path}/{part}: gathered plane table column {k} differs"
             assert (tables["planes"]["plane"].view(np.uint32) == ref["table"]["plane"].view(np.uint32)).all()
         sent = sum(g["exch"]["sent"] for g in gathered)
-        assert all(g["exch"]["mode"] == ("fused-p2p" if mode == "fused" else mode) for g in gathered), [g["exch"]["mode"] for g in gathered]
-        print(f"[multi_gpu_check] world {world} exchange {mode} partition {part}: OK - {len(ref['before'])} blocks, {len(ref['planes'])} "
-              f"fitted planes, {sent} points crossed ranks, shares {[g['exch']['received'] for g in gathered]}; p2p disabled reason: "
-              f"{_PeerBuffers.disabled_reason} / {_FusedExchange.disabled_reason}", flush=True)
+        mode = "fused-p2p" if path == "fused" else "nccl"
+        assert all(g["exch"]["mode"] == mode for g in gathered), [g["exch"]["mode"] for g in gathered]
+        print(f"[multi_gpu_check] world {world} exchange {path} ({mode}) partition {part}: OK - {len(ref['before'])} blocks, "
+              f"{len(ref['planes'])} fitted planes, {sent} points crossed ranks, shares {[g['exch']['received'] for g in gathered]}; "
+              f"fused exchange disabled reason: {gathered[0]['exch']['disabled_reason']}", flush=True)
 dist.barrier()
 dist.destroy_process_group()
