@@ -228,6 +228,17 @@ int ol_forest_map_leaves(ol_forest *f, int32_t op, double param, const int32_t *
 int ol_forest_export_shape(ol_forest *f, int64_t *q, uint32_t *depth, uint64_t *path, int64_t *out_n);
 int ol_forest_impose_shape(ol_forest *f, const int64_t *q, const uint32_t *depth, const uint64_t *path, int64_t n);
 
+/* ---- Grid.locate_points (no counterpart in the reference, whose only way is insert_points of a new pose) ----------
+ * The leaf every query point would be routed into by inserting it as a new pose under the current scheme (grid.py:72-76
+ * for the cell, octree.py:73-97 level by level for the path), without inserting it: nothing changes.  -1 where a
+ * coordinate is not finite, the cell does not exist (cell coordinates outside the packed key range included), or the
+ * point leaves its node above the leaf (insertion would raise IndexError, octree.py:98).
+ * xyz[n][3] float64; on_device != 0: xyz and out are device pointers and the call is stream-ordered, else host
+ * pointers and the call synchronises.  leaf_to_row (device, int32[L], may be NULL) maps a leaf-table index to the value
+ * written (-1 stays -1); NULL writes the leaf-table index (ol_forest_export_leaves order). */
+int ol_forest_locate(ol_forest *f, const double *xyz, int64_t n, int32_t on_device, const int32_t *leaf_to_row,
+                     int64_t *out);
+
 /* ---- measurement support (bench.py): per-stage CUDA-event timers on the forest's stream -------
  * ol_forest_profile(f, 1) clears and enables the timers; ol_forest_profile_read synchronises, writes
  * one line "stage_name launches total_ms" per stage into buf and clears the records.

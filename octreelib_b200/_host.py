@@ -34,6 +34,7 @@ class ForestHost:
         # exports blocks / points in that order; the host only needs the pose epochs for `non_empty=False` listings.
         self._n_subdivides = 0
         self._pose_epoch: Dict[int, int] = {}  # pose index -> subdivide calls made before the pose was created
+        self._rows_cache = (-1, {})  # (forest version, {pose index: leaf -> row table on the device}) for locate
 
     # ---- plumbing --------------------------------------------------------------------------------
     @property
@@ -378,6 +379,47 @@ class ForestHost:
         cov = np.asarray(s["cov"], dtype=np.float64)[:, [0, 1, 2, 1, 3, 4, 2, 4, 5]].reshape(-1, 3, 3)
         return dict(n=np.asarray(s["n"], dtype=np.int64), mean=np.array(s["mean"], dtype=np.float64), covariance=cov,
                     extent=np.array(s["extent"], dtype=np.float64), pose=numbers[np.asarray(s["pose"], dtype=np.int64)])
+
+    # ---- point location ------------------------------------------------------------------------------
+    def locate(self, points, pose_number: Optional[int] = None):
+        """Leaf of every query point of an (n, 3) array (Grid.locate_points): its index in the leaf table, or with a pose
+        number its row of `get_leaf_points(pose_number)`; -1 where there is none.  numpy in -> numpy out, a CUDA tensor
+        in -> int64 CUDA tensor out."""
+        if pose_number is not None and pose_number not in self.pose_index:
+            raise KeyError(pose_number)
+        on_device = bool(getattr(points, "is_cuda", False))
+        if not on_device:
+            points = np.asarray(points)
+        shape = tuple(points.shape)
+        if len(shape) != 2 or shape[1] != 3:
+            raise ValueError(f"points must have shape (n, 3), got {shape}")
+        n = shape[0]
+        if self.empty or n == 0:
+            if on_device:
+                import torch
+
+                return torch.full((n,), -1, dtype=torch.int64, device=points.device)
+            return np.full(n, -1, dtype=np.int64)
+        rows = None if pose_number is None else self._leaf_rows(self.pose_index[pose_number])
+        return self.forest.locate(points, rows)
+
+    def _leaf_rows(self, pose_index: int):
+        """leaf-table index -> row of the pose's non-empty leaves (-1: no point of the pose there), from the block table
+        of the current forest version; uploaded once per (version, pose)"""
+        forest = self.forest
+        version, cache = self._rows_cache
+        if version != forest.version:
+            cache = {}
+            self._rows_cache = (forest.version, cache)
+        rows = cache.get(pose_index)
+        if rows is None:
+            t = _views.tables(forest)
+            blocks = t["blocks"]
+            table = np.full(len(t["leaves"]["edge"]), -1, dtype=np.int32)
+            sel = np.flatnonzero(blocks["pose"] == pose_index)
+            table[blocks["leaf"][sel]] = np.arange(len(sel), dtype=np.int32)
+            rows = cache[pose_index] = forest.upload(table)
+        return rows
 
     # ---- counters (grid.py:343-362) --------------------------------------------------------------
     def counts(self) -> np.ndarray:

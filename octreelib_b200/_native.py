@@ -91,6 +91,7 @@ SIGNATURES = {
     "ol_forest_apply_mask": (C.c_int, [_p]),
     "ol_forest_apply_pose_mask": (C.c_int, [_p, _p, _i32, _p, _i64]),
     "ol_forest_map_leaves": (C.c_int, [_p, _i32, _f64, _p, _i32, _p]),
+    "ol_forest_locate": (C.c_int, [_p, _p, _i64, _i32, _p, _p]),
     "ol_forest_profile": (C.c_int, [_p, _i32]),
     "ol_forest_profile_read": (C.c_int, [_p, C.c_char_p, _i64, C.POINTER(_i64)]),
     "ol_launch_count": (_u64, []),

@@ -351,6 +351,14 @@ int ol_forest_map_leaves(ol_forest* f, int32_t op, double param, const int32_t* 
     OL_API_END
 }
 
+int ol_forest_locate(ol_forest* f, const double* xyz, int64_t n, int32_t on_device, const int32_t* leaf_to_row, int64_t* out) {
+    OL_NEED(f);
+    OL_API_BEGIN
+    ForestScope scope(f->impl);
+    f->impl.locate(xyz, n, on_device != 0, leaf_to_row, out);
+    OL_API_END
+}
+
 int ol_forest_profile(ol_forest* f, int32_t enable) {
     OL_NEED(f);
     OL_API_BEGIN

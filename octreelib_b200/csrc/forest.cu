@@ -1124,5 +1124,6 @@ __global__ void pos_keep_from_block_kernel(uint32_t n, const uint32_t* __restric
 }  // namespace ol
 
 #include "leaf_maps.cuh"
+#include "locate.cuh"
 #include "forest_host.inl"
 #include "forest_host2.inl"

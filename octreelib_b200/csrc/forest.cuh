@@ -273,6 +273,8 @@ struct Forest {
     void apply_pose_mask(const int32_t* pose_rank, int pose, const uint8_t* mask_host, int64_t n);
     // declarative leaf maps (leaf_maps.cuh, ol_forest_map_leaves); rows_appended: NULL or [n_poses]
     void map_leaves(int op, double param, const int32_t* poses, int n_poses_listed, int64_t* rows_appended);
+    // leaf of every query point (locate.cuh, ol_forest_locate); leaf_to_row: NULL or device int32[L]
+    void locate(const double* xyz, int64_t n, bool on_device, const int32_t* leaf_to_row, int64_t* out);
     void pose_counts(int64_t* out_host);
     void stats(ol_forest_stats* s, bool light = false);
     std::string profile_report();  // "name count total_ms" per line; clears the records

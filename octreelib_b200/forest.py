@@ -399,6 +399,30 @@ class Forest:
         self.version += 1
         return rows
 
+    # ---- queries that change nothing -------------------------------------------------------------
+    def locate(self, points, leaf_to_row=None):
+        """Leaf-table index of every query point of an (n, 3) array, or leaf_to_row[index] (an int32 CUDA tensor from
+        `upload`), -1 where no leaf takes the point (`ol_forest_locate`).  numpy in -> int64 numpy out; a CUDA tensor in ->
+        int64 CUDA tensor out, enqueued on the forest's stream (the queries stay on the device)."""
+        if getattr(points, "is_cuda", False) and points.device != self.device:
+            raise ValueError(f"query points are on {points.device}, the grid on {self.device}")
+        table = None if leaf_to_row is None else C.c_void_p(leaf_to_row.data_ptr())
+        with self._scope():
+            src, n, on_dev, _keep = self._as_source(points)  # (a converted tensor is allocated on the forest's stream)
+            if on_dev:
+                out = self._torch.empty(n, dtype=self._torch.int64, device=self.device)
+                dst = C.c_void_p(out.data_ptr())
+            else:
+                out = np.empty(n, dtype=np.int64)
+                dst = _ptr(out)
+            N.check(self._lib.ol_forest_locate(self._h, src, n, on_dev, table, dst))
+        return out
+
+    def upload(self, table: np.ndarray):
+        """A host table as a CUDA tensor on the forest's device (for `locate`'s leaf_to_row)."""
+        with self._scope():
+            return self._torch.from_numpy(np.ascontiguousarray(table)).to(self.device)
+
     # ---- measurement ---------------------------------------------------------------------------
     def profile(self, enable: bool = True):
         with self._scope():

@@ -120,6 +120,32 @@ class Grid(GridBase):
         This is the per-(pose, leaf) hand-off of a plane-based back end (count, centroid, covariance)."""
         return self._host.leaf_statistics(pose_number)
 
+    def leaf_table(self) -> dict:
+        """Every leaf of the current tree shape, empty ones included, as numpy arrays in the reference's leaf enumeration
+        (cells lexicographic, inside a cell the leaf order of a grid subdivided once): `corner` (L, 3) float64, `edge` (L,)
+        float64, `depth` (L,) int32 and `cell` (L, 3) int64, the integer cell coordinates.  `locate_points` without a
+        pose number indexes this table."""
+        host = self._host
+        if host.empty:
+            return dict(corner=np.zeros((0, 3)), edge=np.zeros(0), depth=np.zeros(0, np.int32), cell=np.zeros((0, 3), np.int64))
+        from .. import _views
+
+        t = _views.tables(host.forest)
+        leaves = t["leaves"]
+        return dict(corner=np.array(leaves["corner"], dtype=np.float64), edge=np.array(leaves["edge"], dtype=np.float64),
+                    depth=np.array(leaves["depth"], dtype=np.int32),
+                    cell=np.asarray(t["cells"]["q"], dtype=np.int64)[np.asarray(leaves["cell"], dtype=np.int64)])
+
+    def locate_points(self, points, pose_number: Optional[int] = None):
+        """The leaf every point of an (n, 3) array would be inserted into by `insert_points` of a new pose, computed on
+        the GPU without inserting anything.  Without a pose number: the index into `leaf_table()`; with one: the row of
+        `get_leaf_points(pose_number)` (= the row of `leaf_statistics(pose_number)`), -1 where that pose has no point in
+        the leaf.  -1 also marks a point whose cell does not exist, a non-finite point, and a point insertion would
+        reject (outside its node above the leaf).  numpy in -> int64 numpy out; a CUDA tensor in -> int64 CUDA tensor
+        out on the same device, ordered on the grid's stream.  An unknown pose is a KeyError, a shape other than
+        (n, 3) a ValueError."""
+        return self._host.locate(points, pose_number)
+
     # ---- grid.py:234-242 ------------------------------------------------------------------------
     def get_points(self, pose_number: int) -> PointCloud:
         return self._host.points_dict_order(pose_number)
